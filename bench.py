@@ -2,6 +2,7 @@
 """Benchmark of the NCF training hot path (BASELINE.json metric: NeuMF train samples/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 Workload at N=1: BASELINE.json configs[3] — NeuMF (factor 32, 3 tower layers: 256->128->64->32)
 on the synthetic MovieLens-20M shape (138 493 users x 26 744 items, ~20M interactions, 4
@@ -295,8 +296,49 @@ def config_dict(workload, n_gpus, partitioned=True, tail=False):
                   "exceeds the 126 MB L2 and every step uses a different batch; no explicit flush"}
 
 
+DUMP_ROWS = 16384       # embedding rows written per table by --dump-outputs (a fixed, seeded sample)
+
+
+def dump_outputs(out_dir, ts, loss_before, user, item, label):
+    """--dump-outputs: what the timed steps hand to their caller after the last one, as DIR/<name>.npy, so that
+    two builds can be compared output for output (the inputs are seeded: same arguments, same inputs).
+      loss                    float64 [1]  the loss the caller pops: the per-batch mean losses of the timed steps, summed
+      <state_dict key>        float32      the parameters after the last step, flushed (every row at the Adam state of
+                                           that step); of each embedding table the rows listed in rows_user / rows_item
+      rows_user, rows_item    float64      the sampled row ids (DUMP_ROWS per table, seed 0, ascending)
+      batch_user, batch_item  float64      the batch the last step trained on, as the epoch stream laid it out
+      batch_label             float32
+    Two runs of one build agree bit for bit on the batch and to ~2e-6 relative on the loss, but their parameters
+    only to a median of 1e-6 .. 1e-4 of each array's largest magnitude (B200, default workload, 125 steps in all):
+    the tcgen05 weight-gradient kernel sums in a run-dependent order and Adam amplifies gradients near zero.
+    Compare builds with bounds of that kind (share of elements beyond a tolerance), not element by element."""
+    import numpy as np
+    import torch
+    ts.flush()
+    model = ts.model
+    rng = np.random.default_rng(0)
+    rows = {}
+    for side, n in (("user", model.user_num), ("item", model.item_num)):
+        rows[side] = np.sort(rng.choice(n, size=min(n, DUMP_ROWS), replace=False))
+    arrays = {"loss": (ts.loss_accum - loss_before).cpu().numpy(),
+              "rows_user": rows["user"].astype(np.float64), "rows_item": rows["item"].astype(np.float64),
+              "batch_user": user.cpu().numpy().astype(np.float64), "batch_item": item.cpu().numpy().astype(np.float64),
+              "batch_label": label.cpu().numpy().astype(np.float32)}
+    for k, v in model.state_dict().items():
+        side = "user" if k.startswith("embed_user") else "item" if k.startswith("embed_item") else None
+        if side is not None:
+            v = v[torch.from_numpy(rows[side]).to(v.device)]
+        arrays[k] = v.detach().float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs would write {total} bytes"
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", a)
+
+
 # ------------------------------------------------------------------------------------------------
-def row_sharded_run(dev, world, rank, steps, warmup, tower_math, hbm_peak):
+def row_sharded_run(dev, world, rank, steps, warmup, tower_math, hbm_peak, dump_dir=None):
     """BASELINE configs[4]: NeuMF f=64 L=3 on 10M users x 1M items with the four tables (and their Adam
     state) row-sharded over the ranks; every rank draws `B` samples of its own users per step and item
     rows travel by all-to-all (ncf_b200.dist.RowShardedTrainer).  At N=1 the tables live on the one GPU
@@ -329,6 +371,7 @@ def row_sharded_run(dev, world, rank, steps, warmup, tower_math, hbm_peak):
     sl = lambda k: slice(k * B, (k + 1) * B)
     for k in range(warmup):
         step(bu[sl(k)], bi[sl(k)], bl[sl(k)])
+    loss_before = tr.loss_accum.clone() if dump_dir else None
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
@@ -341,6 +384,9 @@ def row_sharded_run(dev, world, rank, steps, warmup, tower_math, hbm_peak):
         dist.barrier()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if dump_dir:
+        last = sl(warmup + steps - 1)
+        dump_outputs(dump_dir, tr, loss_before, bu[last], bi[last], bl[last])
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -388,7 +434,7 @@ def run_ours(args):
     K, W = args.steps, max(4, args.warmup)     # >= 4: two eager steps, then each of the two step graphs replayed once
 
     if args.workload == "big":
-        res = row_sharded_run(dev, world, rank, K, W, args.tower_math, hbm_peak)
+        res = row_sharded_run(dev, world, rank, K, W, args.tower_math, hbm_peak, args.dump_outputs)
         if rank == 0:
             line = {**res, "higher_is_better": True, "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                     "e2e": None, "gpu_launches": (17 if world > 1 else 8) * K, "roofline": None, "cpu_baseline": None}
@@ -568,6 +614,7 @@ def main_workload(args, dev, world, rank, local, hbm_peak, peak_src, K, W):
         run_window(0, W)
         run_window(1, W)
     T0 = W + (2 * G if wgraphs is not None else 0)     # first timed step
+    loss_before = ts.loss_accum.clone() if args.dump_outputs else None
     sampler = ClockSampler(local)
     sampler.start()     # BEFORE the barrier: nvmlInit takes a different time on every rank, and a rank that enters the
     barrier()           # timed region late is waited for by all the others at the first exchange of the window
@@ -591,6 +638,12 @@ def main_workload(args, dev, world, rank, local, hbm_peak, peak_src, K, W):
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs:
+        if wgraphs is not None:     # the last window's buffers; its last B samples are the last step's batch
+            last = [t[(G - 1) * B:] for t in wbufs[(K // G - 1) & 1]]
+        else:
+            last = bufs[(W + K - 1) & 1]
+        dump_outputs(args.dump_outputs, ts, loss_before, *last)
     value = world * K * B / (ms_total * 1e-3)
     dense = ts.dense_adam(B * world)
     umma = B >= 8192 and f >= 32
@@ -1123,7 +1176,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="end-to-end steps launched eagerly instead of as a CUDA graph")
     ap.add_argument("--tower-math", choices=["fp32", "tf32"], default="fp32",
                     help="fp32 = 3xTF32 parity mode (headline); tf32 = single-pass opt-in mode")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the outputs of --impl ours on one GPU")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -68,7 +68,30 @@ def make_batches(rng, U, I, B, T, hot_users=None):
     return user.astype(np.int64), item.astype(np.int64), label
 
 
-def train_case(NCF, name, model_type, U, I, f, L, B, T, optimizer, lr, seed, short_last=0):
+THIN_BLOCK = 16
+
+
+def thin_outputs(data, L, seed):
+    """Keeps a fixture with a wide tower under 1 MB: of each tower weight matrix in the output groups
+    (grad0, after1, final) one row per block of THIN_BLOCK rows is kept, at a seeded offset inside the
+    block, and the others are stored as NaN (tests/util.py:group masks them out of the comparisons).
+    The inputs stay whole; after2, which no test reads, is dropped."""
+    rng = np.random.default_rng(seed)
+    for k in range(L):
+        key = f"MLP_layers.{3 * k + 1}.weight"
+        rows = data[f"init/{key}"].shape[0]
+        keep = np.arange(0, rows, THIN_BLOCK) + rng.integers(0, THIN_BLOCK, -(-rows // THIN_BLOCK))
+        drop = np.ones(rows, dtype=bool)
+        drop[keep[keep < rows]] = False
+        for prefix in ("grad0", "after1", "final"):
+            a = data[f"{prefix}/{key}"].copy()
+            a[drop] = np.nan
+            data[f"{prefix}/{key}"] = a
+    for k in [k for k in data if k.startswith("after2/")]:
+        del data[k]
+
+
+def train_case(NCF, name, model_type, U, I, f, L, B, T, optimizer, lr, seed, short_last=0, thin=False):
     torch.manual_seed(seed)
     rng = np.random.default_rng(seed)
     model = NCF(U, I, f, L, 0.0, model_type)
@@ -97,6 +120,8 @@ def train_case(NCF, name, model_type, U, I, f, L, B, T, optimizer, lr, seed, sho
             data.update(sd_np(model, "after2"))
     data.update(sd_np(model, "final"))
     data["loss"] = np.array(losses, dtype=np.float64)
+    if thin:
+        thin_outputs(data, L, seed)
     meta = dict(model_type=model_type, U=U, I=I, f=f, L=L, B=B, T=T, optimizer=optimizer, lr=lr,
                 short_last=short_last, torch=torch.__version__)
     np.savez_compressed(OUT / f"{name}.npz", meta=json.dumps(meta), **data)
@@ -271,7 +296,7 @@ def main():
     train_case(NCF, "train_neumf_f32_l2", "NeuMF-end", 50, 30, 32, 2, 48, 6, "adam", 1e-3, 4)
     train_case(NCF, "train_neumf_f6_l2", "NeuMF-end", 33, 21, 6, 2, 20, 6, "adam", 1e-3, 5)
     train_case(NCF, "train_neumf_f5_l1", "NeuMF-end", 33, 21, 5, 1, 20, 5, "adam", 2e-3, 6)
-    train_case(NCF, "train_neumf_f64_l3", "NeuMF-end", 24, 18, 64, 3, 40, 3, "adam", 1e-3, 7)
+    train_case(NCF, "train_neumf_f64_l3", "NeuMF-end", 24, 18, 64, 3, 40, 3, "adam", 1e-3, 7, thin=True)
     train_case(NCF, "train_neumf_f8_l3_sgd", "NeuMF-end", 60, 40, 8, 3, 32, 5, "sgd", 0.01, 8)
     kd_case(NCF, ResponseDistillation, "kd_response", 9)
     pretrain_case(NCF, "neumf_pre_sgd", 10)
