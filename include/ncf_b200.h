@@ -395,6 +395,39 @@ int ncf_eval_users(const NcfModel* m_host, const int64_t* users, const int64_t* 
                    int32_t* topk_idx, float* scores_out, void* workspace, int64_t workspace_bytes,
                    void* stream);
 
+/* ---- full-catalog recommendation and full-ranking evaluation ---------------------------------------
+ * New capability (the reference ranks only the sampled candidates of metrics()).
+ * ncf_mask_items excludes items from per-row scores: for row r, every col[j], j in
+ * [rowptr[users[r]], rowptr[users[r]+1]), with 0 <= col[j] < C sets scores[r, col[j]] = NaN.  A row whose
+ * users[r] is outside [0, user_num) is set to NaN entirely.  rowptr/col: the sorted CSR of ncf_csr_build
+ * (duplicates allowed). */
+int ncf_mask_items(float* scores, int64_t n, int64_t C, const int64_t* users, int64_t user_num,
+                   const int64_t* rowptr, const int32_t* col, void* stream);
+
+/* Per row of scores [n, C]: the k best candidates, best first.  NaN = not a candidate.  Order: larger score
+ * first; equal scores (-0.0 == +0.0) -> lower column first (the rule of ncf_eval_rank).  topk_item[r, j] is
+ * the column, topk_score[r, j] the score as stored in the row.  Rows with fewer than k candidates are padded
+ * with item -1 / score NaN.  target (nullable, [n]): target_rank[r] = number of candidates that precede
+ * column target[r] in that order (full rank, not capped by k); -1 when the target is outside [0, C), not a
+ * candidate, or target is NULL (target_rank nullable only then).  1 <= k <= 1024, k <= C < 2^31.
+ * Every score is read four times whatever k is (radix select in shared memory: the workspace query returns 0
+ * for valid arguments, -1 otherwise). */
+int64_t ncf_topk_rows_workspace_bytes(int64_t n, int64_t C, int32_t k);
+int ncf_topk_rows(const float* scores, int64_t n, int64_t C, int32_t k, const int64_t* target,
+                  int64_t* topk_item, float* topk_score, int32_t* target_rank,
+                  void* workspace, int64_t workspace_bytes, void* stream);
+
+/* Scores users[0..n) against every item of the model (the forward kernels of ncf_forward), excludes each
+ * user's CSR row (rowptr/col with user_num + 1 row pointers; both NULL: no exclusion) and selects as
+ * ncf_topk_rows, with columns = item ids.  Users are processed min(chunk_users, n) at a time, at most 2^28
+ * (user, item) pairs per chunk: workspace = scores [chunk, item_num] + item ids [chunk * item_num] + forward
+ * workspace, sized by ncf_recommend_workspace_bytes(m, min(chunk_users, n), k).  k <= item_num < 2^31. */
+int64_t ncf_recommend_workspace_bytes(const NcfModel* m, int64_t chunk_users, int32_t k);
+int ncf_recommend(const NcfModel* m, const int64_t* users, int64_t n, int32_t k,
+                  const int64_t* rowptr, const int32_t* col, const int64_t* target, int64_t chunk_users,
+                  int64_t* topk_item, float* topk_score, int32_t* target_rank,
+                  void* workspace, int64_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

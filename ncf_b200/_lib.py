@@ -109,6 +109,11 @@ SIGNATURES = {
     "ncf_eval_rank": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "ncf_eval_workspace_bytes": (_i64, [_P(NcfModel), _i64, _i32]),
     "ncf_eval_users": (C.c_int, [_P(NcfModel), _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ncf_mask_items": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp]),
+    "ncf_topk_rows_workspace_bytes": (_i64, [_i64, _i64, _i32]),
+    "ncf_topk_rows": (C.c_int, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ncf_recommend_workspace_bytes": (_i64, [_P(NcfModel), _i64, _i32]),
+    "ncf_recommend": (C.c_int, [_P(NcfModel), _vp, _i64, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 
 LIB_PATH = Path(__file__).resolve().parent / "libncf_b200.so"

@@ -90,6 +90,20 @@ int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t 
   return launch_mma_forward(p, tower_passes(m), st);
 }
 
+// Workspace of forward_dispatch for any batch up to p.B (with p.user_div as the caller will pass it).
+int64_t forward_workspace_bytes(const TileParams& p) {
+  const int64_t B = p.B;
+  int64_t bytes = mma_tile_rows(p) ? align_up(mma_split_floats(p) * 4, 256) : 0;
+  if (umma_eligible(p))
+    bytes = std::max(bytes, align_up(umma_forward_workspace_floats(p, B) * 4, 256) + 256);
+  // any batch up to B may be passed with a workspace of this size: cover the small-batch path as well
+  TileParams ps = p;
+  ps.B = std::min<int64_t>(B, 2048);
+  if (ps.B > 0 && wide_eligible(ps))
+    bytes = std::max(bytes, align_up(wide_workspace_floats(ps, ps.B) * 4, 256));
+  return bytes;
+}
+
 }  // namespace ncf
 
 extern "C" int64_t ncf_forward_workspace_bytes(const NcfModel* m, int64_t B) {
@@ -97,15 +111,7 @@ extern "C" int64_t ncf_forward_workspace_bytes(const NcfModel* m, int64_t B) {
   TileParams p{};
   ncf::fill_model_params(p, m);
   p.B = B;
-  int64_t bytes = ncf::mma_tile_rows(p) ? ncf::align_up(ncf::mma_split_floats(p) * 4, 256) : 0;
-  if (ncf::umma_eligible(p))
-    bytes = std::max(bytes, ncf::align_up(ncf::umma_forward_workspace_floats(p, B) * 4, 256) + 256);
-  // any batch up to B may be passed with a workspace of this size: cover the small-batch path as well
-  TileParams ps = p;
-  ps.B = std::min<int64_t>(B, 2048);
-  if (ps.B > 0 && ncf::wide_eligible(ps))
-    bytes = std::max(bytes, ncf::align_up(ncf::wide_workspace_floats(ps, ps.B) * 4, 256));
-  return bytes;
+  return ncf::forward_workspace_bytes(p);
 }
 
 extern "C" int ncf_forward(const NcfModel* m, const int64_t* user, const int64_t* item, int64_t B,

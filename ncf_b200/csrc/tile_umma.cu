@@ -1758,8 +1758,13 @@ int64_t umma_scratch_floats(const TileParams& p, int64_t B, bool train) {
 
 constexpr int64_t kForwardSub = 262144;  // inference sub-batch: bounds the activation scratch
 
+// rows of one inference sub-batch: a whole number of users when one user covers user_div rows
+static int64_t forward_sub(const TileParams& p) {
+  return p.user_div > 0 ? std::max<int64_t>(1, kForwardSub / p.user_div) * p.user_div : kForwardSub;
+}
+
 int64_t umma_forward_workspace_floats(const TileParams& p, int64_t B) {
-  return umma_image_floats(p) + umma_scratch_floats(p, std::min<int64_t>(B, kForwardSub), false) + 64;
+  return umma_image_floats(p) + umma_scratch_floats(p, std::min<int64_t>(B, forward_sub(p)), false) + 64;
 }
 int64_t umma_train_workspace_floats(const TileParams& p, int64_t B) {
   return umma_image_floats(p) + umma_scratch_floats(p, B, true) + 64;
@@ -1789,8 +1794,7 @@ int launch_umma_forward(TileParams& p, int passes, float* ws, cudaStream_t st) {
     if (rc != NCF_OK) return rc;
     return launch_tower<false>(p, passes, st);
   }
-  int64_t sub = kForwardSub;
-  if (p.user_div > 0) sub = std::max<int64_t>(1, sub / p.user_div) * p.user_div;
+  const int64_t sub = forward_sub(p);
   carve(p, ws, std::min(B, sub), false, st, &rc);
   if (rc != NCF_OK) return rc;
   const int64_t* user = p.user;

@@ -59,6 +59,24 @@ def evaluate_top_k(model, users: torch.Tensor, cands: torch.Tensor, max_k: int =
     return hr_at_k, ndcg_at_k
 
 
+def evaluate_full_ranking(model, users: torch.Tensor, targets: torch.Tensor, exclude, ks=(1, 5, 10, 20)):
+    """Full-ranking leave-one-out protocol: the held-out item targets[r] is ranked against every item user
+    users[r] has not seen (exclude = (rowptr, col) of ops.csr_build over the training pairs), ties to the
+    lower item id.  One ncf_recommend pass (k = 1: only the target's rank is needed).
+    Returns (rank int32 [n] on the device, -1 = target excluded; {K: HR@K}; {K: NDCG@K}), means over users
+    with NDCG = 1/log2(rank+2) in float64 as EvalResult.lists() computes it."""
+    from .recommend import recommend_ranked
+    _, _, rank = recommend_ranked(model, users, 1, exclude, target=targets)
+    r = rank.cpu().numpy().astype(np.int64)
+    gain = np.where(r >= 0, 1.0 / np.log2(np.maximum(r, 0) + 2.0), 0.0)
+    hr_at_k, ndcg_at_k = {}, {}
+    for k in ks:
+        hit = (r >= 0) & (r < k)
+        hr_at_k[k] = float(np.mean(hit.astype(np.float64))) if r.size else 0.0
+        ndcg_at_k[k] = float(np.mean(np.where(hit, gain, 0.0))) if r.size else 0.0
+    return rank, hr_at_k, ndcg_at_k
+
+
 def evaluate_top_k_performance(model, test_loader, max_k=10):
     """Drop-in for reference scripts/evaluate_models.py:22-32 (same name, arguments and return value)."""
     device = next(model.parameters()).device

@@ -566,6 +566,102 @@ def eval_users(m: NcfModel, users: torch.Tensor, cands: torch.Tensor, k: int):
     return hit, rank, ndcg, topk, scores
 
 
+# ---- full-catalog recommendation ------------------------------------------------------------------------
+def _caller_workspace(workspace: Optional[torch.Tensor], ws_bytes: int, what: str, device):
+    if workspace is None:
+        return _workspace(device, ws_bytes)
+    if workspace.numel() * workspace.element_size() < ws_bytes:
+        raise _lib.NcfError(f"{what}: workspace of {workspace.numel() * workspace.element_size()} bytes "
+                            f"is smaller than the {ws_bytes} needed")
+    return workspace
+
+
+def mask_items(scores: torch.Tensor, users: torch.Tensor, rowptr: torch.Tensor, col: torch.Tensor) -> torch.Tensor:
+    """In place: scores[r, c] = NaN for every item c of user users[r]'s CSR row (rowptr, col of csr_build);
+    rows of users outside the CSR are NaN entirely.  Returns scores."""
+    if scores.dim() != 2 or scores.shape[0] != users.numel():
+        raise _lib.NcfError("mask_items: scores must be [n, C] with one row per user")
+    if col.dtype != torch.int32:
+        raise _lib.NcfError(f"col must be int32, got {col.dtype}")
+    n, Cc = scores.shape
+    colp = col if col.numel() else torch.zeros(1, dtype=torch.int32, device=scores.device)
+    check(_lib.load().ncf_mask_items(ptr(_f32(scores, "scores")), n, Cc, ptr(_i64(users, "users")),
+                                     rowptr.numel() - 1, ptr(_i64(rowptr, "rowptr")), ptr(colp), current_stream()),
+          "ncf_mask_items")
+    return scores
+
+
+def topk_rows(scores: torch.Tensor, k: int, target: Optional[torch.Tensor] = None,
+              workspace: Optional[torch.Tensor] = None):
+    """scores [n, C] (NaN = not a candidate) -> (items int64 [n, k], scores f32 [n, k], target_rank int32 [n]
+    or None): the k best columns of every row, larger score first, ties to the lower column, rows with fewer
+    candidates padded with -1 / NaN; target_rank = the full rank of column target[r] (-1: not a candidate)."""
+    lib = _lib.load()
+    if scores.dim() != 2:
+        raise _lib.NcfError("topk_rows: scores must be [n, C]")
+    n, Cc = scores.shape
+    dev = scores.device
+    ws_bytes = int(lib.ncf_topk_rows_workspace_bytes(n, Cc, k))
+    if ws_bytes < 0:
+        raise _lib.NcfError(f"topk_rows: k={k} outside [1, min(1024, C={Cc})]")
+    ws = _caller_workspace(workspace, ws_bytes, "topk_rows", dev)
+    items = torch.empty(n, k, dtype=torch.int64, device=dev)
+    top = torch.empty(n, k, dtype=torch.float32, device=dev)
+    rank = None
+    if target is not None:
+        if target.numel() != n:
+            raise _lib.NcfError("topk_rows: target must hold one column per row")
+        rank = torch.empty(n, dtype=torch.int32, device=dev)
+    check(lib.ncf_topk_rows(ptr(_f32(scores, "scores")), n, Cc, k,
+                            ptr(_i64(target, "target")) if target is not None else None, ptr(items), ptr(top),
+                            ptr(rank), ptr(ws), ws_bytes, current_stream()), "ncf_topk_rows")
+    return items, top, rank
+
+
+def recommend_workspace_bytes(m: NcfModel, chunk_users: int, k: int) -> int:
+    n = int(_lib.load().ncf_recommend_workspace_bytes(C.byref(m), chunk_users, k))
+    if n < 0:
+        raise _lib.NcfError(f"ncf_recommend_workspace_bytes: bad model, k={k} or chunk_users={chunk_users}")
+    return n
+
+
+def recommend(m: NcfModel, users: torch.Tensor, k: int, chunk_users: int, rowptr: Optional[torch.Tensor] = None,
+              col: Optional[torch.Tensor] = None, target: Optional[torch.Tensor] = None,
+              workspace: Optional[torch.Tensor] = None):
+    """Scores users [n] against every item of the model, excludes each user's CSR row (rowptr, col of
+    csr_build; None: no exclusion) and selects as topk_rows: -> (items int64 [n, k], scores f32 [n, k],
+    target_rank int32 [n] or None).  `workspace`: caller-owned scratch of recommend_workspace_bytes(m,
+    min(chunk_users, n), k) bytes (required for calls that end up in a CUDA graph)."""
+    lib = _lib.load()
+    n, dev = users.numel(), users.device
+    if (rowptr is None) != (col is None):
+        raise _lib.NcfError("recommend: rowptr and col go together")
+    if rowptr is not None:
+        if col.dtype != torch.int32:
+            raise _lib.NcfError(f"col must be int32, got {col.dtype}")
+        if rowptr.numel() != m.user_num + 1:
+            raise _lib.NcfError(f"recommend: rowptr has {rowptr.numel()} entries, the model {m.user_num} users")
+        if not col.numel():
+            col = torch.zeros(1, dtype=torch.int32, device=dev)
+    items = torch.empty(n, k, dtype=torch.int64, device=dev)
+    top = torch.empty(n, k, dtype=torch.float32, device=dev)
+    rank = None
+    if target is not None:
+        if target.numel() != n:
+            raise _lib.NcfError("recommend: target must hold one item per user")
+        rank = torch.empty(n, dtype=torch.int32, device=dev)
+    if n == 0:
+        return items, top, rank
+    ws_bytes = recommend_workspace_bytes(m, min(int(chunk_users), n), k)
+    ws = _caller_workspace(workspace, ws_bytes, "recommend", dev)
+    check(lib.ncf_recommend(C.byref(m), ptr(_i64(users, "users")), n, k,
+                            ptr(_i64(rowptr, "rowptr")) if rowptr is not None else None, ptr(col),
+                            ptr(_i64(target, "target")) if target is not None else None, int(chunk_users),
+                            ptr(items), ptr(top), ptr(rank), ptr(ws), ws.numel() * ws.element_size(),
+                            current_stream()), "ncf_recommend")
+    return items, top, rank
+
+
 # ---- (e) row-sharded tables -------------------------------------------------------------------------------
 def train_step_grads_norm(m: NcfModel, g: NcfGrads, user, item, label, B_norm: int,
                           loss_accum: torch.Tensor, workspace: torch.Tensor, teacher_logits=None,
