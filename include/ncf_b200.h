@@ -297,7 +297,10 @@ int ncf_adam_step_dense(const NcfModel* m_host, const NcfGrads* g_host, const Nc
  * those user rows - the other user rows are never read or written on this rank.  parts: mask of 1 (user
  * tables), 2 (item tables), 4 (tower) = what this call updates; the rest was updated by another path of
  * the same step (the peer-memory exchange ncf_adam_p2p for the replicated item tables and the tower).
- * Every row of both sides is stamped as current and the step counter is incremented whatever parts is. */
+ * Whatever parts is, user rows [user_lo, user_hi) and every item row are stamped as current (last step =
+ * the new step, flags cleared), the step counter is incremented and the touched counts are zeroed; user rows
+ * outside the range are not touched.  Gradients are consumed (zeroed) only in the parts updated.  Partial
+ * parts need row widths that are multiples of 4 floats. */
 int ncf_adam_step_dense_range(const NcfModel* m_host, const NcfGrads* g_host, const NcfAdamState* s_host,
                               NcfAdamHyper h, int64_t user_lo, int64_t user_hi, int32_t parts, void* stream);
 /* Optimiser sharding for replicated data parallelism (new design, SURVEY.md 8e): with parameters,
@@ -344,7 +347,9 @@ int ncf_sgd_step(const NcfModel* m_host, const NcfGrads* g_host, float lr, void*
  * local index r / world.
  * ncf_bucket_by_owner: groups the n samples by the owner of their item: perm[pos] = sample index,
  *   local_idx[pos] = item / world, counts[w] = samples whose item lives on rank w; cursor is
- *   int32[world] scratch.  ncf_permute_*: out[i] = in[perm[i]].
+ *   int32[world] scratch.  A negative item (ncf_sample_neg's -1) counts for owner 0 with local_idx = -1, so
+ *   counts and perm still cover all n samples; ncf_gather_rows zero-fills its row and ncf_scatter_add_rows
+ *   skips it.  1 <= world <= 64.  ncf_permute_*: out[i] = in[perm[i]].
  * ncf_gather_rows: out[i][:] = table[idx[i]][:].  ncf_scatter_add_rows: table[idx[i]][:] += in[i][:]. */
 int ncf_bucket_by_owner(const int64_t* item, int64_t n, int32_t world, int64_t* perm,
                         int64_t* local_idx, int32_t* counts, int32_t* cursor, void* stream);

@@ -8,7 +8,8 @@
 #include <cuda_runtime.h>
 
 // Zero-gradient steps replayed exactly per row.  The per-step term decays like
-// (b1/sqrt(b2))^j ~ 0.9005^j, so what is dropped beyond 160 steps is < 1e-7 of the first term.
+// (b1/sqrt(b2))^j ~ 0.9005^j times the change of the bias corrections, so what is dropped beyond 160 steps
+// sums to < 1.4e-6 of the first term (worst for a row last stepped at step 12; DESIGN §3.2).
 constexpr int kMaxReplay = 160;
 
 struct AdamConst {

@@ -10,6 +10,11 @@ namespace {
 
 constexpr int kMaxWorld = 64;
 
+// Owner of an item row.  A negative id (ncf_sample_neg writes -1 for a user without a legal negative) is
+// given to rank 0 with local index -1, which ncf_gather_rows zero-fills and ncf_scatter_add_rows skips;
+// `it % world` would be negative there and index outside the histogram and the cursor array.
+__device__ __forceinline__ int owner_of(int64_t it, int world) { return it < 0 ? 0 : (int)(it % world); }
+
 __global__ void owner_count_kernel(const int64_t* __restrict__ item, int64_t n, int world,
                                    int32_t* __restrict__ counts) {
   __shared__ int32_t h[kMaxWorld];
@@ -17,7 +22,7 @@ __global__ void owner_count_kernel(const int64_t* __restrict__ item, int64_t n, 
   __syncthreads();
   for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < n;
        b += (int64_t)gridDim.x * blockDim.x)
-    atomicAdd(&h[(int)(item[b] % world)], 1);
+    atomicAdd(&h[owner_of(item[b], world)], 1);
   __syncthreads();
   for (int i = threadIdx.x; i < world; i += blockDim.x)
     if (h[i]) atomicAdd(&counts[i], h[i]);
@@ -33,16 +38,16 @@ __global__ void owner_scan_kernel(const int32_t* __restrict__ counts, int world,
 }
 
 // perm[pos] = sample index, grouped by owner (order inside a group is arbitrary);
-// local_idx[pos] = item / world of that sample.
+// local_idx[pos] = item / world of that sample (-1 for a negative item).
 __global__ void owner_place_kernel(const int64_t* __restrict__ item, int64_t n, int world,
                                    int32_t* __restrict__ cursor, int64_t* __restrict__ perm,
                                    int64_t* __restrict__ local_idx) {
   for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < n;
        b += (int64_t)gridDim.x * blockDim.x) {
     const int64_t it = item[b];
-    const int pos = atomicAdd(&cursor[(int)(it % world)], 1);
+    const int pos = atomicAdd(&cursor[owner_of(it, world)], 1);
     perm[pos] = b;
-    local_idx[pos] = it / world;
+    local_idx[pos] = it < 0 ? -1 : it / world;
   }
 }
 
