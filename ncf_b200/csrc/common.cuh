@@ -80,6 +80,24 @@ __device__ __forceinline__ float4 ldg4(const float* p) {
   return __ldg(reinterpret_cast<const float4*>(p));
 }
 
+// The per-sample training objective, defined once for every tile kernel and loss_grad_kernel (the KD
+// objective of distill.cu is a different one): BCE-with-logits of logit x against label y, mixed with
+// the squared distance to the teacher logit t when there is a teacher (alpha weights the BCE term).
+// `loss` is the sample's term of the batch sum; `dlogit` is d(mean loss)/dx, i.e. already scaled by
+// invB = 1 / batch size.
+struct SampleLoss {
+  float loss, dlogit;
+};
+__device__ __forceinline__ SampleLoss sample_loss(float x, float y, bool has_teacher, float t, float alpha,
+                                                  float invB) {
+  const float e = expf(-fabsf(x));
+  const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
+  const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
+  if (!has_teacher) return {bce, (sig - y) * invB};
+  const float df = x - t;
+  return {alpha * bce + (1.f - alpha) * df * df, (alpha * (sig - y) + (1.f - alpha) * 2.f * df) * invB};
+}
+
 // 16-byte vector reduction into global memory (RED.E.ADD.F32x4 on sm_90+).
 __device__ __forceinline__ void red_add4(float* p, float4 v) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y),

@@ -135,12 +135,12 @@ __global__ void step_tail_kernel(const StepTail tail) { step_tail(tail, *tail.st
 template <int MODE>
 __device__ __forceinline__ void adam_rows_body(const RowsParams& q, int64_t step_now);
 
-// TAIL (mode 0 only): the step ends here (step_tail)
-template <int MODE, bool TAIL = false>
+// mode 0 ends the step (step_tail); the other modes ignore `tail`
+template <int MODE>
 __global__ void __launch_bounds__(kThreads) adam_rows_kernel(const RowsParams q, const StepTail tail) {
   const int64_t step_now = *q.step;
   adam_rows_body<MODE>(q, step_now);
-  if (TAIL) step_tail(tail, step_now);
+  if (MODE == 0) step_tail(tail, step_now);
 }
 
 template <int MODE>
@@ -662,16 +662,8 @@ static int adam_step_impl(const NcfModel* m, const NcfGrads* g, const NcfAdamSta
     step_tail_kernel<<<32, 256, 0, st>>>(tail);
     NCF_LAUNCH_CHECK("step_tail_kernel");
   } else {
-    static const bool fold = [] { const char* e = getenv("NCF_STEP_TAIL"); return !(e && e[0] == '0'); }();
-    if (fold) {
-      adam_rows_kernel<0, true><<<rows_grid(g_rows_hint), kThreads, 0, st>>>(q, tail);
-      NCF_LAUNCH_CHECK("adam_rows_kernel");
-    } else {
-      adam_rows_kernel<0, false><<<rows_grid(g_rows_hint), kThreads, 0, st>>>(q, StepTail{});
-      NCF_LAUNCH_CHECK("adam_rows_kernel");
-      step_tail_kernel<<<8, 256, 0, st>>>(tail);
-      NCF_LAUNCH_CHECK("step_tail_kernel");
-    }
+    adam_rows_kernel<0><<<rows_grid(g_rows_hint), kThreads, 0, st>>>(q, tail);
+    NCF_LAUNCH_CHECK("adam_rows_kernel");
   }
   g_rows_hint = 0;
   return NCF_OK;

@@ -13,20 +13,11 @@ __global__ void loss_grad_kernel(const float* __restrict__ logits, const float* 
   float ls = 0.f;
   for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < B;
        b += (int64_t)gridDim.x * blockDim.x) {
-    const float x = logits[b], y = label[b];
-    const float e = expf(-fabsf(x));
-    const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-    const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-    float dl;
-    if (teacher != nullptr) {
-      const float df = x - teacher[b];
-      ls += alpha * bce + (1.f - alpha) * df * df;
-      dl = (alpha * (sig - y) + (1.f - alpha) * 2.f * df) * invB;
-    } else {
-      ls += bce;
-      dl = (sig - y) * invB;
-    }
-    if (dlogit != nullptr) dlogit[b] = dl;
+    float t = 0.f;
+    if (teacher != nullptr) t = teacher[b];
+    const SampleLoss r = sample_loss(logits[b], label[b], teacher != nullptr, t, alpha, invB);
+    ls += r.loss;
+    if (dlogit != nullptr) dlogit[b] = r.dlogit;
   }
   __shared__ float part[32];
   ls = warp_sum(ls);

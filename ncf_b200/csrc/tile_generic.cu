@@ -188,19 +188,10 @@ __global__ void __launch_bounds__(kThreads) ncf_tile_kernel(const TileParams p) 
           if (ok && p.dlogit_in != nullptr) {
             dl = p.dlogit_in[b];
           } else if (ok) {
-            const float y = p.label[b];
-            const float e = expf(-fabsf(x));
-            const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-            const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-            if (p.teacher != nullptr) {
-              const float t = p.teacher[b];
-              const float df = x - t;
-              ls = p.alpha * bce + (1.f - p.alpha) * df * df;
-              dl = (p.alpha * (sig - y) + (1.f - p.alpha) * 2.f * df) * p.invB;
-            } else {
-              ls = bce;
-              dl = (sig - y) * p.invB;
-            }
+            const bool kd = p.teacher != nullptr;
+            const SampleLoss r = sample_loss(x, p.label[b], kd, kd ? p.teacher[b] : 0.f, p.alpha, p.invB);
+            ls = r.loss;
+            dl = r.dlogit;
           }
           dl_s[m] = dl;
           ls_s[m] = ls;

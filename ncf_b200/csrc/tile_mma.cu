@@ -18,34 +18,8 @@
 // embedding-row gradients leave the CTA as vector REDs (dW_k is small and L2-resident).
 //
 // Replaces reference src/ncf/models.py:97-118 and scripts/train_neumf.py:112-114.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tile_params.cuh"
-
-#ifdef NCF_PHASE_TIMING
-__device__ unsigned long long g_phase_cycles[16];
-#define NCF_PHASE(i)                                                            \
-  do {                                                                          \
-    __syncthreads();                                                            \
-    if (blockIdx.x == 0 && threadIdx.x == 0) {                                  \
-      const long long now = clock64();                                          \
-      g_phase_cycles[i] += (unsigned long long)(now - phase_t0);                \
-      phase_t0 = now;                                                           \
-    }                                                                           \
-  } while (0)
-extern "C" int ncf_debug_phase_cycles(unsigned long long* out_host, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(out_host, g_phase_cycles, sizeof(g_phase_cycles));
-  if (reset) {
-    unsigned long long z[16] = {0};
-    cudaMemcpyToSymbol(g_phase_cycles, z, sizeof(z));
-  }
-  return 0;
-}
-#else
-#define NCF_PHASE(i) do {} while (0)
-#endif
 
 namespace {
 
@@ -402,9 +376,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
   for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int64_t base = tile * TM;
     __syncthreads();
-#ifdef NCF_PHASE_TIMING
-    long long phase_t0 = clock64();
-#endif
     if (tid < TM) {
       const int64_t b = base + tid;
       int64_t u = -1, it = -1;
@@ -453,7 +424,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
     cp_async_commit();
     cp_async_wait<0>();
     __syncthreads();
-    NCF_PHASE(0);  // indices + gather
 
     // ---- tower forward ------------------------------------------------------------------------------
     if (has_mlp) {
@@ -474,7 +444,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
       }
     }
     __syncthreads();
-    NCF_PHASE(1);  // tower forward
 
     // ---- predict layer: one warp per sample row computes the logit ------------------------------------------
     const float* hL = act(L);
@@ -506,18 +475,10 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
         if (ok && p.dlogit_in != nullptr) {
           dl = p.dlogit_in[b];
         } else if (ok) {
-          const float y = p.label[b];
-          const float e = expf(-fabsf(x));
-          const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-          const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-          if (p.teacher != nullptr) {
-            const float df = x - p.teacher[b];
-            ls = p.alpha * bce + (1.f - p.alpha) * df * df;
-            dl = (p.alpha * (sig - y) + (1.f - p.alpha) * 2.f * df) * p.invB;
-          } else {
-            ls = bce;
-            dl = (sig - y) * p.invB;
-          }
+          const bool kd = p.teacher != nullptr;
+          const SampleLoss r = sample_loss(x, p.label[b], kd, kd ? p.teacher[b] : 0.f, p.alpha, p.invB);
+          ls = r.loss;
+          dl = r.dlogit;
         }
         dl_s[m] = dl;
         ls_s[m] = ls;
@@ -584,7 +545,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
     }
     __syncthreads();
     for (int c = tid; c < p.predict_size; c += kThreads) atomicAdd(&p.gt[p.pw_off + c], pg_s[c]);
-    NCF_PHASE(2);  // predict, loss, predict grads, GMF scatter
 
     // ---- tower backward ----------------------------------------------------------------------------------------
     if (has_mlp) {
@@ -597,7 +557,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
         }
       }
       __syncthreads();
-      NCF_PHASE(3);  // GMF scatter + delta_L
       for (int k = L - 1; k >= 0; --k) {
         const int K = p.W[k], N = p.W[k + 1];
         const float* dn = act(k + 1);  // delta_{k+1} [TM][N]
@@ -615,11 +574,9 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
             atomicAdd(&p.gt[p.b_off[k] + n], s);
           }
         }
-        NCF_PHASE(4);  // bias gradients
         // weight gradient
         wgrad_dispatch<PASSES, TM>(dn, ldd, N, act(k), lda(k), K, p.gt + p.w_off[k]);
         __syncthreads();  // every read of H_k is done before it is overwritten by delta_k
-        NCF_PHASE(5 + min(k, 2));  // wgrad of layer k (5: k=0, 6: k=1, 7: k>=2)
         float* hk = act(k);
         const int ldh = lda(k);
         for (int c0 = 0; c0 < K; c0 += kStageRows) {
@@ -643,7 +600,6 @@ __global__ void __launch_bounds__(kThreads, 1) ncf_mma_tile_kernel(const TilePar
           }
         }
         __syncthreads();
-        NCF_PHASE(8 + min(k, 2));  // backward data of layer k (8: dX, 9: k=1, 10: k>=2)
       }
     }
   }
@@ -691,15 +647,10 @@ namespace ncf {
 
 // 0 = not eligible, else the tile height (64 or 32).
 int mma_tile_rows(const TileParams& p_in) {
-  static const int min_f = getenv("NCF_MMA_MIN_F") ? atoi(getenv("NCF_MMA_MIN_F")) : 8;  // tuning knob
-  if (p_in.f < min_f) return 0;
   if (p_in.type == NCF_GMF) return 0;          // no tower: the generic kernel is already a pure gather
   if (p_in.f < 8 || (p_in.f & (p_in.f - 1)) != 0) return 0;  // block shapes assume power-of-two widths
   TileParams p = p_in;
   const bool fit64 = mma_smem_bytes<64>(p) <= kSmemLimit, fit32 = mma_smem_bytes<32>(p) <= kSmemLimit;
-  static const int forced = getenv("NCF_MMA_TILE_ROWS") ? atoi(getenv("NCF_MMA_TILE_ROWS")) : 0;  // tuning knob
-  if (forced == 64 && fit64) return 64;
-  if (forced == 32 && fit32) return 32;
   // a batch that leaves most SMs idle with 64-row tiles (the reference's 256: 4 CTAs) runs on twice as many CTAs
   if (fit32 && p.B > 0 && (p.B + 63) / 64 * 2 <= ncf::num_sms()) return 32;
   if (fit64) return 64;

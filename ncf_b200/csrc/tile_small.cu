@@ -14,8 +14,6 @@
 //
 // Replaces reference src/ncf/models.py:97-118 (forward), scripts/train_neumf.py:112-114 (criterion + backward)
 // and src/distillation/base.py:40-50 + response.py:28-32 (KD loss) for these shapes.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tile_params.cuh"
 
@@ -238,18 +236,10 @@ __global__ void __launch_bounds__(kThreads) ncf_small_tile_kernel(const TilePara
     if (ok && p.dlogit_in != nullptr) {
       dl = p.dlogit_in[row];
     } else if (ok) {
-      const float y = p.label[row];
-      const float e = expf(-fabsf(x));
-      const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-      const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-      if (p.teacher != nullptr) {
-        const float df = x - p.teacher[row];
-        ls = p.alpha * bce + (1.f - p.alpha) * df * df;
-        dl = (p.alpha * (sig - y) + (1.f - p.alpha) * 2.f * df) * p.invB;
-      } else {
-        ls = bce;
-        dl = (sig - y) * p.invB;
-      }
+      const bool kd = p.teacher != nullptr;
+      const SampleLoss r = sample_loss(x, p.label[row], kd, kd ? p.teacher[row] : 0.f, p.alpha, p.invB);
+      ls = r.loss;
+      dl = r.dlogit;
     }
     if (warp == 0) {
       const float ls_w = warp_sum(ls), dl_w = warp_sum(dl);
@@ -347,8 +337,7 @@ namespace ncf {
 
 // factor_num 8, 1..3 tower layers, MLP / NeuMF (GMF has no tower: the generic kernel is a pure gather)
 bool small_eligible(const TileParams& p) {
-  static const bool off = getenv("NCF_SMALL_DISABLE") != nullptr && getenv("NCF_SMALL_DISABLE")[0] == '1';
-  if (off || p.f != kF || p.type == NCF_GMF || p.L < 1 || p.L > 3) return false;
+  if (p.f != kF || p.type == NCF_GMF || p.L < 1 || p.L > 3) return false;
   for (int k = 0; k < p.L; ++k)
     if (reinterpret_cast<uintptr_t>(p.w[k]) & 15) return false;   // weights are staged with 16-byte loads
   return true;

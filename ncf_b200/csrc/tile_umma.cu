@@ -24,8 +24,6 @@
 //
 // Layouts, issue rates and hand-off costs were measured on this hardware first: tools/umma_probe.cu,
 // tools/mma_issue_probe.cu, tools/sync_probe.cu (outputs and the kernel's phase trace in profiles/).
-// Debug aids compiled out by default: -DNCF_UMMA_TRACE (clock64 timeline of CTA 0), NCF_UMMA_ABLATE
-// (knock-outs of single ingredients, results are wrong, only the time matters).
 #include <algorithm>
 #include <cstdlib>
 
@@ -51,7 +49,6 @@ struct GemmArgs {
   int layer;    // tower layer index k
   int gather;   // A rows are [embed_user_MLP[u] | embed_item_MLP[i]] instead of a dense matrix
   int stages;
-  int ablate;   // debugging knock-outs (NCF_UMMA_ABLATE bit mask), 0 in production
   const float* a;      // dense A [B][K]
   const float* b_img;  // weight image: [panel][hi|lo][n_total rows][32]
   const float* bias;
@@ -64,7 +61,7 @@ struct WgradJob {
   int S;  // samples per stage: scaled so that every job moves the same bytes per hand-off
 };
 struct WgradArgs {
-  int njobs, passes, ablate;
+  int njobs, passes;
   WgradJob job[12];
 };
 
@@ -231,14 +228,6 @@ __global__ void umma_weight_images_kernel(const TileParams p) {
   }
 }
 
-#ifdef NCF_UMMA_TRACE
-// timeline of CTA 0 (debug builds only): clock64 at the hand-off points of each role
-__device__ long long g_trace[3][128];
-#define NCF_TRACE(role, slot) do { if (blockIdx.x == 0 && blockIdx.y == 0 && (slot) < 128) g_trace[role][slot] = clock64(); } while (0)
-#else
-#define NCF_TRACE(role, slot) do { } while (0)
-#endif
-
 // ---- GEMM kernel ------------------------------------------------------------------------------------
 struct GemmBars {
   uint64_t full[kMaxStages], empty[kMaxStages], acc_full[2], acc_empty[2];
@@ -338,7 +327,7 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
       for (int j = 0; j < 2; ++j) {
         const int r = r0 + 64 * j;
         const float* src = nullptr;
-        if (ok[j] && !(g.ablate & 1)) src = g.gather ? (c0 < d ? src_u[j] + c0 : src_i[j] + (c0 - d)) : src_u[j] + c0;
+        if (ok[j]) src = g.gather ? (c0 < d ? src_u[j] + c0 : src_i[j] + (c0 - d)) : src_u[j] + c0;
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           const int piece = 2 * c + hq;
@@ -353,13 +342,11 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
       if (is_s >= g.stages) { is_s -= g.stages; is_ph ^= 1; }
       return true;
     };
-    int tr = 0;
     auto consume = [&](bool more_pending) {
       if (more_pending) asm volatile("cp.async.wait_group 1;" ::: "memory");
       else asm volatile("cp.async.wait_group 0;" ::: "memory");
-      if (u == 0 && grp == 0) NCF_TRACE(0, tr);
       uint8_t* st = smem + (size_t)cs * stage_bytes;
-      if (g.passes == 3 && !(g.ablate & 16)) {
+      if (g.passes == 3) {
 #pragma unroll
         for (int j = 0; j < 2; ++j) {
           const int r = r0 + 64 * j;
@@ -373,8 +360,6 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
         }
       }
       fence_async_smem();
-      if (u == 0 && grp == 0) NCF_TRACE(0, tr + 1);
-      tr += 2;
       mbar_arrive_warp(&bars.full[cs]);
       cs += 2;
       if (cs >= g.stages) cs -= g.stages;
@@ -400,9 +385,7 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
         mbar_wait(&bars.empty[s], ph ^ 1);
         uint8_t* st = smem + (size_t)s * stage_bytes;
         const float* bsrc = g.b_img + (int64_t)pi * 2 * g.n_total * 32 + (int64_t)nb * N * 32;
-        if (g.ablate & 2) {
-          mbar_arrive(&bars.full[s]);
-        } else if (g.passes == 3) {
+        if (g.passes == 3) {
           mbar_expect_tx(&bars.full[s], 2 * b_bytes);
           bulk_g2s(st + 2 * a_bytes, bsrc, b_bytes, &bars.full[s]);
           bulk_g2s(st + 2 * a_bytes + b_bytes, bsrc + (int64_t)g.n_total * 32, b_bytes, &bars.full[s]);
@@ -419,7 +402,7 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
     if (lane == 0) {
       const uint32_t idesc = make_idesc(kTile, N, 0, 0);
       uint32_t lt = 0, ph = 0;
-      int s = 0, tr = 0;
+      int s = 0;
       for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++lt) {
         const int a = lt & 1;
         mbar_wait(&bars.acc_empty[a], ((lt >> 1) & 1) ^ 1);
@@ -427,11 +410,10 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
         const uint32_t d_tmem = tmem + a * N;
         for (int pi = 0; pi < panels; ++pi) {
           mbar_wait(&bars.full[s], ph);
-          NCF_TRACE(1, tr);
           tc_fence_after();
           const uint32_t base = smem_u32(smem + (size_t)s * stage_bytes);
           const uint32_t ahi = base, alo = base + a_bytes, bhi = base + 2 * a_bytes, blo = bhi + b_bytes;
-          const int ksteps = (g.ablate & 4) ? 0 : min(4, (K - pi * 32) >> 3);
+          const int ksteps = min(4, (K - pi * 32) >> 3);
           for (int ks = 0; ks < ksteps; ++ks) {
             const uint64_t dah = make_desc(ahi + ks * 32, 16, 1024, 2);
             const uint64_t dbh = make_desc(bhi + ks * 32, 16, 1024, 2);
@@ -444,8 +426,6 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
             }
           }
           tc_commit(&bars.empty[s]);
-          NCF_TRACE(1, tr + 1);
-          tr += 2;
           if (++s == g.stages) { s = 0; ph ^= 1; }
         }
         tc_commit(&bars.acc_full[a]);
@@ -463,17 +443,11 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
       const int a = lt & 1;
       if (a != grp) continue;
       mbar_wait_warp(&bars.acc_full[a], (lt >> 1) & 1);
-      if (q == 0 && lane == 0) NCF_TRACE(2, 2 * (int)lt);
       tc_fence_after();
       const int64_t row = tile * kTile + q * 32 + lane;
       const bool valid = row < p.B;
       const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16) + a * N;
       float v[32];
-      if (g.ablate & 8) {
-        tc_fence_before();
-        mbar_arrive_warp(&bars.acc_empty[a]);
-        continue;
-      }
 
       if (EPI == EPI_RELU_STORE) {
         float* out = g.out + row * (int64_t)g.n_total + nb * N;
@@ -557,18 +531,10 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
           if (ok && p.dlogit_in != nullptr) {
             dl = p.dlogit_in[row];
           } else if (ok) {
-            const float y = p.label[row];
-            const float e = expf(-fabsf(x));
-            const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-            const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-            if (p.teacher != nullptr) {
-              const float df = x - p.teacher[row];
-              ls = p.alpha * bce + (1.f - p.alpha) * df * df;
-              dl = (p.alpha * (sig - y) + (1.f - p.alpha) * 2.f * df) * p.invB;
-            } else {
-              ls = bce;
-              dl = (sig - y) * p.invB;
-            }
+            const bool kd = p.teacher != nullptr;
+            const SampleLoss r = sample_loss(x, p.label[row], kd, kd ? p.teacher[row] : 0.f, p.alpha, p.invB);
+            ls = r.loss;
+            dl = r.dlogit;
           }
           const float ls_w = warp_sum(ls), dl_w = warp_sum(dl);
           if (lane == 0) {
@@ -620,7 +586,6 @@ umma_gemm_kernel(const __grid_constant__ TileParams p, const __grid_constant__ G
         }
       }
       tc_fence_before();
-      if (q == 0 && lane == 0) NCF_TRACE(2, 2 * (int)lt + 1);
       mbar_arrive_warp(&bars.acc_empty[a]);
     }
   }
@@ -661,7 +626,7 @@ struct TowerGemm {
   const float* img;
 };
 struct TowerArgs {
-  int passes, ng, ablate;
+  int passes, ng;
   int ring_col, ring_stages;
   int hcol[NCF_MAX_LAYERS + 1], lcol[NCF_MAX_LAYERS + 1];
   TowerGemm gemm[kMaxGemms];
@@ -787,7 +752,7 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
     int s = grp;            // ring stage of the next own panel (flat over tiles: P0 is even)
     uint32_t ph = 0;
     auto copy_panel = [&](int64_t tl, int pi, int64_t uu, int64_t ii) {
-      const bool ok = tl < my_tiles && uu >= 0 && uu < p.U && ii >= 0 && ii < p.I && !(g.ablate & 1);
+      const bool ok = tl < my_tiles && uu >= 0 && uu < p.U && ii >= 0 && ii < p.I;
       const int c0 = pi * 32;
       const float* src = p.eum;
       if (ok) src = (c0 < d) ? p.eum + uu * d + c0 : p.eim + ii * d + (c0 - d);
@@ -818,7 +783,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
       mbar_wait_warp(&bars.tile_done, (uint32_t)tl & 1);
       for (int pi = grp; pi < P0; pi += 2) {
         // pending groups: the rest of this tile's own panels, then the next tile's first ones
-        if (warp == 0 && lane == 0 && tl == 1) NCF_TRACE(0, 4 * (pi / 2));
         if (own == 4) asm volatile("cp.async.wait_group 3;" ::: "memory");
         else if (own == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
         else asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -829,9 +793,7 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
           const float4 x = *reinterpret_cast<const float4*>(src + ((c ^ (r & 7)) << 4));
           cur[4 * c] = x.x; cur[4 * c + 1] = x.y; cur[4 * c + 2] = x.z; cur[4 * c + 3] = x.w;
         }
-        if (warp == 0 && lane == 0 && tl == 1) NCF_TRACE(0, 4 * (pi / 2) + 1);
         mbar_wait_warp(&bars.a_empty[s], ph ^ 1);
-        if (warp == 0 && lane == 0 && tl == 1) NCF_TRACE(0, 4 * (pi / 2) + 2);
         tc_fence_after();
         const uint32_t col = lane_addr + g.ring_col + s * 64;
         tc_st32(col, cur);
@@ -842,7 +804,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
         }
         tc_wait_st();
         tc_fence_before();
-        if (warp == 0 && lane == 0 && tl == 1) NCF_TRACE(0, 4 * (pi / 2) + 3);
         mbar_arrive_warp(&bars.a_full[s]);
         // refill the slot this thread has just read with the next tile's row - after the hand-off:
         // the copies would otherwise sit in front of it in the warp's memory-instruction queue
@@ -908,9 +869,7 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
             mbar_wait(&bars.b_empty[s], ph ^ 1);
             const float* src = G.img + (int64_t)pi * 2 * G.n_total * 32 + (int64_t)G.row0 * 32;
             uint8_t* dst = smem + (size_t)s * b_stage;
-            if (g.ablate & 2) {
-              mbar_arrive(&bars.b_full[s]);
-            } else if (G.N == G.n_total) {  // hi and lo of the panel are contiguous
+            if (G.N == G.n_total) {  // hi and lo of the panel are contiguous
               mbar_expect_tx(&bars.b_full[s], bytes);
               bulk_g2s(dst, src, bytes, &bars.b_full[s]);
             } else {
@@ -942,7 +901,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
             ++n_opnd;
             tc_fence_after();
           }
-          if (pass == 0 && set == 0) NCF_TRACE(1, 2 * ((int)tl * g.ng + gi));
           for (int pi = 0; pi < panels; ++pi, ++n_panel) {
             if ((int)(n_panel % kTowerMmaSets) != set) {  // the other set's panel: only keep the ring cursors in step
               if (G.a_hi >= 0 && G.new_operand) ppar ^= 1u << pi;
@@ -953,7 +911,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
             uint32_t a_hi, a_lo;
             if (G.a_hi < 0) {
               mbar_wait(&bars.a_full[sa], pha);
-              if (pass == 0 && set == 0 && tl == 1) NCF_TRACE(2, 64 + 3 * pi);
               a_hi = tmem + g.ring_col + sa * 64;
               a_lo = a_hi + 32;
             } else {
@@ -965,28 +922,23 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
               a_lo = tmem + G.a_lo + pi * 32;
             }
             mbar_wait(&bars.b_full[sb], phb);
-            if (pass == 0 && set == 0 && tl == 1 && gi == 0) NCF_TRACE(2, 64 + 3 * pi + 1);
             tc_fence_after();
             const uint32_t bhi = smem_u32(smem + (size_t)sb * b_stage);
             // the k-step only moves the start-address field of the descriptor (32 B = 2 units of 16 B)
             const uint64_t dbh0 = make_desc(bhi, 16, 1024, 2);
             const uint64_t dbl0 = make_desc(bhi + (uint32_t)G.N * 128, 16, 1024, 2);
-            if (!(g.ablate & 4)) {
-              const uint32_t a_op = (pass == 1) ? a_lo : a_hi;
-              const uint64_t b_op = (pass == 2) ? dbl0 : dbh0;
+            const uint32_t a_op = (pass == 1) ? a_lo : a_hi;
+            const uint64_t b_op = (pass == 2) ? dbl0 : dbh0;
 #pragma unroll
-              for (int ks = 0; ks < 4; ++ks) tc_mma_ts(d_tmem, a_op + ks * 8, b_op + 2 * ks, idesc, 1u);
-            }
+            for (int ks = 0; ks < 4; ++ks) tc_mma_ts(d_tmem, a_op + ks * 8, b_op + 2 * ks, idesc, 1u);
             if (G.a_hi < 0) {
               tc_commit(&bars.a_empty[sa]);
               if (++sa == NA) { sa = 0; pha ^= 1; }
             }
             tc_commit(&bars.b_empty[sb]);
-            if (pass == 0 && set == 0 && tl == 1 && gi == 0) NCF_TRACE(2, 64 + 3 * pi + 2);
             if (++sb == kBStages) { sb = 0; phb ^= 1; }
           }
           tc_commit(&bars.acc_ready[gi & 1]);
-          if (pass == 0 && set == 0) NCF_TRACE(1, 2 * ((int)tl * g.ng + gi) + 1);
         }
     }
   } else {
@@ -1049,7 +1001,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
         }
         mbar_wait_warp(&bars.acc_ready[gi & 1], n_acc[gi & 1] & 1);
         ++n_acc[gi & 1];
-        if (warp == kTowerEpiWarp0 + 1 && lane == 0) NCF_TRACE(2, 2 * ((int)tl * g.ng + gi));
         tc_fence_after();
         // published only now: the accumulator of this tile's last layer is ready, so its layer-0 panels
         // have been supplied, so gather group 0 is done reading the previous tile's dlogit from xch[]
@@ -1076,31 +1027,11 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
         const int nchunk = N >> 5;
         const int c_begin = (nchunk >= 2) ? hf * (nchunk / 2) * 32 : 0;
         const int c_end = (nchunk >= 2) ? (hf + 1) * (nchunk / 2) * 32 : (hf == 0 ? N : 0);
-        if (g.ablate & 8) {
-          // nothing
-        } else if (G.kind == 0 && k + 1 < L) {
-          // ---- forward layer: X = relu(Z + b) -> scratch, TMEM hi (in place) and lo ------------------------
-          const int kk = k + 1;
-          const float* bias = p.b[k];
-          for (int c0 = c_begin; c0 < c_end; c0 += 32) {
-            tc_ld32(lane_addr + g.hcol[kk] + c0, v);
-#pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j] + __ldg(&bias[c0 + j]), 0.f);
-            tc_st32(lane_addr + g.hcol[kk] + c0, v);
-            if (g.passes == 3) {
-              float lo[32];
-#pragma unroll
-              for (int j = 0; j < 32; ++j) lo[j] = lo_of(v[j]);
-              tc_st32(lane_addr + g.lcol[kk] + c0, lo);
-            }
-            if (TRAIN) quad8_transpose(v, lane);  // shuffle work while the TMEM stores drain
-            tc_wait_st();
-            tc_fence_before();
-            mbar_arrive_warp(&bars.panel_ready[c0 >> 5]);
-            if (TRAIN) store_rows_t(v, p.act[kk], N, row - lane, p.B, c0, lane);
-          }
-
-        } else if (G.kind == 0) {
+        // The branch order steers ptxas' register allocation at the 96-register cap, and was chosen for the
+        // training kernel: with the forward layers first it spills 40 more bytes (996 vs 956).  The
+        // backward-data branches are compiled into the training kernel only (launch_tower<false> queues
+        // forward GEMMs only); in the inference kernel they would cost spills, not just dead code.
+        if (G.kind == 0 && k + 1 == L) {
           // ---- last layer + predict layer (+ loss, predict grads, GMF scatter, delta_L) ---------------------
           // The two warps of a lane quarter split the work: half 0 owns the tower side (logit, loss,
           // delta_L), half 1 the GMF branch (its partial logit was computed before the accumulator was
@@ -1124,18 +1055,9 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
               if (ok && p.dlogit_in != nullptr) {
                 dl = p.dlogit_in[row];
               } else if (ok) {
-                const float y = pre_label;
-                const float e = expf(-fabsf(x));
-                const float bce = fmaxf(x, 0.f) - x * y + log1pf(e);
-                const float sig = (x >= 0.f) ? 1.f / (1.f + e) : e / (1.f + e);
-                if (p.teacher != nullptr) {
-                  const float df = x - pre_teacher;
-                  ls = p.alpha * bce + (1.f - p.alpha) * df * df;
-                  dl = (p.alpha * (sig - y) + (1.f - p.alpha) * 2.f * df) * p.invB;
-                } else {
-                  ls = bce;
-                  dl = (sig - y) * p.invB;
-                }
+                const SampleLoss r = sample_loss(x, pre_label, p.teacher != nullptr, pre_teacher, p.alpha, p.invB);
+                ls = r.loss;
+                dl = r.dlogit;
               }
               bars.xch[trow] = dl;
               mbar_arrive_warp(&bars.dl_ready);  // the GMF-branch gradients are the idle gather warps' job
@@ -1171,7 +1093,29 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
           } else {
             named_bar(1 + q, 64);
           }
-        } else if (k > 0) {
+        } else if (G.kind == 0) {
+          // ---- forward layer: X = relu(Z + b) -> scratch, TMEM hi (in place) and lo ------------------------
+          const int kk = k + 1;
+          const float* bias = p.b[k];
+          for (int c0 = c_begin; c0 < c_end; c0 += 32) {
+            tc_ld32(lane_addr + g.hcol[kk] + c0, v);
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j] + __ldg(&bias[c0 + j]), 0.f);
+            tc_st32(lane_addr + g.hcol[kk] + c0, v);
+            if (g.passes == 3) {
+              float lo[32];
+#pragma unroll
+              for (int j = 0; j < 32; ++j) lo[j] = lo_of(v[j]);
+              tc_st32(lane_addr + g.lcol[kk] + c0, lo);
+            }
+            if (TRAIN) quad8_transpose(v, lane);  // shuffle work while the TMEM stores drain
+            tc_wait_st();
+            tc_fence_before();
+            mbar_arrive_warp(&bars.panel_ready[c0 >> 5]);
+            if (TRAIN) store_rows_t(v, p.act[kk], N, row - lane, p.B, c0, lane);
+          }
+
+        } else if (TRAIN && k > 0) {
           // ---- backward data: dZ_k = dX_k * (X_k > 0) -> scratch, TMEM hi (in place) and lo (over X_k) --------
           for (int c0 = c_begin; c0 < c_end; c0 += 32) {
             float x[32];
@@ -1191,7 +1135,7 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
             mbar_arrive_warp(&bars.panel_ready[c0 >> 5]);
             store_rows_t(v, p.delta[k], N, row - lane, p.B, c0, lane);
           }
-        } else {
+        } else if (TRAIN) {
           // ---- backward data of layer 0: scatter into the embedding-gradient rows -------------------------------
           for (int c0 = c_begin; c0 < c_end; c0 += 32) {
             tc_ld32(lane_addr + G.d_col + c0, v);
@@ -1210,7 +1154,6 @@ umma_tower_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
         if (zero_late) zero_cols(g.gemm[0].d_col, g.gemm[0].N);  // both halves are past the named barrier: the read is over
         tc_wait_st();
         tc_fence_before();
-        if (warp == kTowerEpiWarp0 + 1 && lane == 0) NCF_TRACE(2, 2 * ((int)tl * g.ng + gi) + 1);
         if (gi + 1 == g.ng) mbar_arrive_warp(&bars.tile_done);
       }
     }
@@ -1329,15 +1272,13 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
       const uint32_t par = (uint32_t)((ci / kWgStages) & 1) ^ 1;
       if (blocking) mbar_wait_warp(&bars.empty[s], par);
       else if (!mbar_test_warp(&bars.empty[s], par)) return false;
-      if (t == 0) NCF_TRACE(0, 2 * (int)ci);
       uint8_t* st = smem + (size_t)s * stage_bytes;
       const int64_t row0 = (local + ci * job.nctas) * S;
-      const bool off = (g.ablate & 64) != 0;
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         if (i < na) {
           const int64_t row = row0 + sa0 + i * sas;
-          const bool ok = row < p.B && !off;
+          const bool ok = row < p.B;
           cp_async16_zfill(st + mn_offset(sa0 + i * sas, ca * 4, S),
                            ok ? delta + row * nout + job.mb * 128 + ca * 4 : delta, ok);
         }
@@ -1349,11 +1290,11 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
           bool ok;
           if (k == 0) {
             const int64_t ix = (ci & 1) ? idx_odd[i] : idx_even[i];
-            ok = ix >= 0 && ix < idx_lim && !off;
+            ok = ix >= 0 && ix < idx_lim;
             src = ok ? tab + ix * d : tab;
           } else {
             const int64_t row = row0 + sb0 + i * sbs;
-            ok = row < p.B && !off;
+            ok = row < p.B;
             src = ok ? actk + row * kin + fo : actk;
           }
           cp_async16_zfill(st + 2 * a_img + mn_offset(sb0 + i * sbs, cb * 4, S), src, ok);
@@ -1373,33 +1314,28 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
       else if (newer == 2) asm volatile("cp.async.wait_group 2;" ::: "memory");
       else if (newer == 1) asm volatile("cp.async.wait_group 1;" ::: "memory");
       else asm volatile("cp.async.wait_group 0;" ::: "memory");
-      if (!(g.ablate & 256)) {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          if (i < na) {
-            const uint32_t off = mn_offset(sa0 + i * sas, ca * 4, S);
-            const float4 x = *reinterpret_cast<const float4*>(st + off);
-            float4 hi, lo;
-            split4(x, hi, lo);
-            dbsum.x += x.x; dbsum.y += x.y; dbsum.z += x.z; dbsum.w += x.w;
-            if (g.ablate & 512) *reinterpret_cast<float4*>(st + off) = x;
-            if (g.passes == 3) *reinterpret_cast<float4*>(st + a_img + off) = lo;
-          }
+      for (int i = 0; i < 4; ++i) {
+        if (i < na) {
+          const uint32_t off = mn_offset(sa0 + i * sas, ca * 4, S);
+          const float4 x = *reinterpret_cast<const float4*>(st + off);
+          float4 hi, lo;
+          split4(x, hi, lo);
+          dbsum.x += x.x; dbsum.y += x.y; dbsum.z += x.z; dbsum.w += x.w;
+          if (g.passes == 3) *reinterpret_cast<float4*>(st + a_img + off) = lo;
         }
+      }
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          if (i < nbp && g.passes == 3) {
-            const uint32_t off = 2 * a_img + mn_offset(sb0 + i * sbs, cb * 4, S);
-            const float4 x = *reinterpret_cast<const float4*>(st + off);
-            float4 hi, lo;
-            split4(x, hi, lo);
-            if (g.ablate & 512) *reinterpret_cast<float4*>(st + off) = x;
-            *reinterpret_cast<float4*>(st + b_img + off) = lo;
-          }
+      for (int i = 0; i < 8; ++i) {
+        if (i < nbp && g.passes == 3) {
+          const uint32_t off = 2 * a_img + mn_offset(sb0 + i * sbs, cb * 4, S);
+          const float4 x = *reinterpret_cast<const float4*>(st + off);
+          float4 hi, lo;
+          split4(x, hi, lo);
+          *reinterpret_cast<float4*>(st + b_img + off) = lo;
         }
       }
       fence_async_smem();
-      if (t == 0) NCF_TRACE(0, 2 * (int)ci + 1);
       mbar_arrive_warp(&bars.full[s]);
     };
     if (k == 0) {
@@ -1432,7 +1368,7 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
       float v[32];
       for (int c0 = part * (NB / parts); c0 < (part + 1) * (NB / parts) && part < parts; c0 += 32) {
         tc_ld32(tmem + ((uint32_t)(q * 32) << 16) + c0, v);
-        if (m < MB && !(g.ablate & 32)) {
+        if (m < MB) {
 #pragma unroll
           for (int j = 0; j < 32; j += 4) red_add4(dst + c0 + j, make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]));
         }
@@ -1444,16 +1380,14 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
     for (int64_t ci = 0; ci < my_chunks; ++ci) {
       const int s = (int)(ci % kWgStages);
       mbar_wait(&bars.full[s], (uint32_t)(ci / kWgStages) & 1);
-      if (pass == 0) NCF_TRACE(1, 2 * (int)ci);
       tc_fence_after();
       const uint32_t base = smem_u32(smem + (size_t)s * stage_bytes);
       const uint32_t ahi = base, alo = base + a_img, bhi = base + 2 * a_img, blo = bhi + b_img;
       // the k-step (8 sample rows = 1024 B) only moves the start-address field: +64 units of 16 B
       const uint64_t da0 = make_desc(pass == 1 ? alo : ahi, S * 128, 512, 1);
       const uint64_t db0 = make_desc(pass == 2 ? blo : bhi, S * 128, 512, 1);
-      for (int ks = 0; ks < ((g.ablate & 128) ? 0 : S / 8); ++ks) tc_mma(tmem, da0 + 64 * ks, db0 + 64 * ks, idesc, 1u);
+      for (int ks = 0; ks < S / 8; ++ks) tc_mma(tmem, da0 + 64 * ks, db0 + 64 * ks, idesc, 1u);
       tc_commit(&bars.empty[s]);
-      if (pass == 0) NCF_TRACE(1, 2 * (int)ci + 1);
     }
     if (my_chunks > 0) tc_commit(&bars.acc_full);
   }
@@ -1465,17 +1399,6 @@ umma_wgrad_kernel(const __grid_constant__ TileParams p, const __grid_constant__ 
 // ---- launchers ---------------------------------------------------------------------------------------------
 constexpr size_t kSmemBudget = 200 * 1024;
 
-// debug-only knobs, read once per process (the knobs tests flip at run time - NCF_UMMA_DISABLE, NCF_UMMA_FUSED,
-// NCF_UMMA_MIN_B - are read per call)
-static int ablate_knob() {
-  static const int v = [] { const char* e = getenv("NCF_UMMA_ABLATE"); return e ? atoi(e) : 0; }();
-  return v;
-}
-static bool timing_knob() {
-  static const bool v = getenv("NCF_UMMA_TIMING") != nullptr;
-  return v;
-}
-
 template <int EPI>
 int launch_gemm(const TileParams& p, GemmArgs g, int nblocks, cudaStream_t st) {
   const size_t stage = 2 * (size_t)kTile * 128 + 2 * (size_t)g.N * 128;
@@ -1486,7 +1409,6 @@ int launch_gemm(const TileParams& p, GemmArgs g, int nblocks, cudaStream_t st) {
     return NCF_ERR_ARG;
   }
   g.stages = stages;
-  g.ablate = ablate_knob();
   const size_t smem = stages * stage + 1024;
   auto kern = umma_gemm_kernel<EPI>;
   NCF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1495,31 +1417,12 @@ int launch_gemm(const TileParams& p, GemmArgs g, int nblocks, cudaStream_t st) {
   if (grid > ntiles) grid = ntiles;
   kern<<<dim3((unsigned)grid, (unsigned)nblocks), kGemmThreads, smem, st>>>(p, g);
   NCF_LAUNCH_CHECK("umma_gemm_kernel");
-#ifdef NCF_UMMA_TRACE
-  {
-    static int calls = 0;
-    const char* want = getenv("NCF_UMMA_TRACE_CALL");  // index of the launch to print (counted per process)
-    if (want && atoi(want) == calls) {
-      cudaStreamSynchronize(st);
-      static long long h[3][128];
-      cudaMemcpyFromSymbol(h, g_trace, sizeof(h));
-      const long long t0 = h[0][0];
-      fprintf(stderr, "[trace] EPI=%d K=%d N=%d stages=%d\n", EPI, g.K, g.N, g.stages);
-      for (int i = 0; i < 48; i += 2)
-        fprintf(stderr, "[trace] %2d  prod: empty-ok %7lld stored %7lld | mma: full-ok %7lld committed %7lld | epi(tile %d): acc-ok %7lld done %7lld\n",
-                i / 2, h[0][i] - t0, h[0][i + 1] - t0, h[1][i] - t0, h[1][i + 1] - t0, i / 2,
-                i / 2 < 8 ? h[2][i] - t0 : 0, i / 2 < 8 ? h[2][i + 1] - t0 : 0);
-    }
-    ++calls;
-  }
-#endif
   return NCF_OK;
 }
 
 int launch_wgrad(const TileParams& p, int passes, cudaStream_t st) {
   WgradArgs g{};
   g.passes = passes;
-  g.ablate = ablate_knob();
   // one job per [128 x 256] block of every layer's dW; CTAs shared out by operand bytes per sample
   double weight[12], total = 0;
   for (int k = 0; k < p.L; ++k) {
@@ -1559,23 +1462,12 @@ int launch_wgrad(const TileParams& p, int passes, cudaStream_t st) {
   NCF_CUDA(cudaFuncSetAttribute(umma_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   umma_wgrad_kernel<<<cta, kWgradThreads, smem, st>>>(p, g);
   NCF_LAUNCH_CHECK("umma_wgrad_kernel");
-#ifdef NCF_UMMA_TRACE
-  if (getenv("NCF_UMMA_TRACE_WGRAD")) {
-    cudaStreamSynchronize(st);
-    static long long h[3][128];
-    cudaMemcpyFromSymbol(h, g_trace, sizeof(h));
-    const long long t0 = h[0][0];
-    for (int i = 0; i < 48; i += 2)
-      fprintf(stderr, "[wtrace] %2d  prod: empty-ok %7lld stored %7lld | mma: full-ok %7lld committed %7lld\n", i / 2,
-              h[0][i] - t0, h[0][i + 1] - t0, h[1][i] - t0, h[1][i + 1] - t0);
-  }
-#endif
   return NCF_OK;
 }
 
 // Per-launch CUDA-event times of one training step on the tcgen05 path.  Enabled by
-// ncf_profile_enable(1) (results read back with ncf_profile_read) or NCF_UMMA_TIMING=1 (printed to
-// stderr).  Profiling synchronises the stream after every step: measurement aid, not for production.
+// ncf_profile_enable(1), read back with ncf_profile_read.  Profiling synchronises the stream after
+// every step: measurement aid, not for production.
 struct StepProfile {
   int enabled = 0, n = 0;
   float ms[16];
@@ -1590,7 +1482,7 @@ struct StepTimer {
   const char* name[32];
   int n = 0;
   static thread_local StepTimer* g_timer;
-  StepTimer(cudaStream_t s) : on(g_profile.enabled || timing_knob()), st(s) {
+  StepTimer(cudaStream_t s) : on(g_profile.enabled), st(s) {
     g_timer = this;
     mark("start");
   }
@@ -1608,11 +1500,9 @@ struct StepTimer {
     for (int i = 1; i < n; ++i) {
       float ms = 0;
       cudaEventElapsedTime(&ms, ev[i - 1], ev[i]);
-      if (g_profile.enabled && g_profile.n < 16) {
+      if (g_profile.n < 16) {
         g_profile.ms[g_profile.n] = ms;
         g_profile.name[g_profile.n++] = name[i];
-      } else {
-        fprintf(stderr, "[umma] %-10s %8.1f us\n", name[i], ms * 1e3f);
       }
     }
     for (int i = 0; i < n; ++i) cudaEventDestroy(ev[i]);
@@ -1654,7 +1544,8 @@ int tower_forward(TileParams& p, int passes, bool train, cudaStream_t st) {
   return NCF_OK;
 }
 
-// The fused kernel needs the whole tile's operand chain in the 512 TMEM columns.
+// The fused kernel needs the whole tile's operand chain in the 512 TMEM columns.  NCF_UMMA_FUSED=0 is a
+// test hook that forces the per-layer GEMMs; it is read per call, so a test can switch it between calls.
 bool tower_fused_ok(const TileParams& p) {
   const char* off = getenv("NCF_UMMA_FUSED");
   if (off != nullptr && off[0] == '0') return false;
@@ -1668,7 +1559,6 @@ template <bool TRAIN>
 int launch_tower(const TileParams& p, int passes, cudaStream_t st) {
   TowerArgs g{};
   g.passes = passes;
-  g.ablate = ablate_knob();
   int col = 0;
   for (int k = 1; k <= p.L; ++k) {
     g.hcol[k] = col;
@@ -1700,24 +1590,6 @@ int launch_tower(const TileParams& p, int passes, cudaStream_t st) {
   if (grid > ntiles) grid = ntiles;
   kern<<<(unsigned)grid, kTowerThreads, smem, st>>>(p, g);
   NCF_LAUNCH_CHECK("umma_tower_kernel");
-#ifdef NCF_UMMA_TRACE
-  if (getenv("NCF_UMMA_TRACE_TOWER")) {
-    cudaStreamSynchronize(st);
-    static long long h[3][128];
-    cudaMemcpyFromSymbol(h, g_trace, sizeof(h));
-    const long long t0 = h[1][0];
-    for (int i = 0; i < 4; ++i)
-      fprintf(stderr, "[ptrace] own panel %d: start %7lld landed+read %7lld ring-free %7lld stored %7lld\n", i, h[0][4 * i] - t0,
-              h[0][4 * i + 1] - t0, h[0][4 * i + 2] - t0, h[0][4 * i + 3] - t0);
-    for (int i = 0; i < 8; ++i)
-      fprintf(stderr, "[mtrace] panel %d: a_full %7lld b_full %7lld committed %7lld\n", i, h[2][64 + 3 * i] - t0,
-              h[2][64 + 3 * i + 1] - t0, h[2][64 + 3 * i + 2] - t0);
-    for (int i = 0; i < 2 * g.ng; ++i)
-      fprintf(stderr, "[ttrace] tile %d gemm %d (kind %d k %d N %3d K %3d): mma start %7lld issued %7lld | epi acc-ok %7lld done %7lld\n",
-              i / g.ng, i % g.ng, g.gemm[i % g.ng].kind, g.gemm[i % g.ng].k, g.gemm[i % g.ng].N, g.gemm[i % g.ng].K,
-              h[1][2 * i] - t0, h[1][2 * i + 1] - t0, h[2][2 * i] - t0, h[2][2 * i + 1] - t0);
-  }
-#endif
   return NCF_OK;
 }
 
@@ -1727,6 +1599,8 @@ namespace ncf {
 
 // Eligible: a tower whose widths are power-of-two multiples of 32 (panels of 32 fp32, accumulator
 // chunks of 32 columns) and a batch large enough that ~10 launches beat one fused launch.
+// Test hooks, read per call: NCF_UMMA_DISABLE=1 keeps the path off, NCF_UMMA_MIN_B lowers the batch
+// threshold so that small test batches run it.
 bool umma_eligible(const TileParams& p) {
   const char* off = getenv("NCF_UMMA_DISABLE");
   if (off != nullptr && off[0] == '1') return false;

@@ -12,8 +12,6 @@
 // Replaces reference src/ncf/models.py:97-118 (forward) for these calls; same contract as the other forward
 // kernels (TileParams; tile_params.cuh): out-of-range indices give NaN logits, user_div > 0 = one user per
 // user_div candidates.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tile_params.cuh"
 
@@ -125,8 +123,7 @@ namespace ncf {
 
 // forward only; MLP / NeuMF; every layer input a multiple of 32 wide (factor_num a multiple of 16); small batch
 bool wide_eligible(const TileParams& p) {
-  static const bool off = getenv("NCF_WIDE_DISABLE") != nullptr && getenv("NCF_WIDE_DISABLE")[0] == '1';
-  if (off || p.type == NCF_GMF || p.L < 1 || p.B < 1 || p.B > kWideMaxB) return false;
+  if (p.type == NCF_GMF || p.L < 1 || p.B < 1 || p.B > kWideMaxB) return false;
   if (p.f < 16 || (p.f & 15) != 0 || (p.d & 3) != 0) return false;
   for (int k = 0; k < p.L; ++k)
     if ((p.W[k] & 31) != 0 || (reinterpret_cast<uintptr_t>(p.w[k]) & 15) != 0) return false;
