@@ -387,8 +387,11 @@ int ncf_shard_push_grads(const int64_t* item, int64_t n, int32_t world, int64_t 
 /* ---- a11: leave-one-out evaluation --------------------------------------------------------------
  * Replaces metrics() (reference src/training/metrics.py:4-25).  scores is [n, C]; column 0 is the
  * held-out positive (reference src/data/datasets.py:31-34).  Per user: topk_idx[k] = indices of the
- * k largest scores in descending order, ties broken towards the LOWER candidate index; rank =
- * position of candidate 0 in that order (or -1); hit = rank >= 0; ndcg = 1/log2(rank+2) or 0.
+ * k largest scores in descending order, ties (-0.0 == +0.0) broken towards the LOWER candidate index;
+ * NaN is not a candidate, and a row with fewer than k non-NaN scores is padded with -1.  This is the
+ * order of ncf_topk_rows.  rank = position of candidate 0 in that order, or -1 when it is not among
+ * the first k or is NaN; hit = rank >= 0; ndcg = 1/log2(rank+2) or 0.  (torch.topk, which the
+ * reference uses, ranks NaN above every number, so there a NaN held-out score counts as a hit.)
  * Any of hit / rank / ndcg / topk_idx may be NULL.  Requires 1 <= k <= C <= 1024. */
 int ncf_eval_rank(const float* scores, int64_t n, int32_t C, int32_t k, uint8_t* hit,
                   int32_t* rank, float* ndcg, int32_t* topk_idx, void* stream);

@@ -13,7 +13,9 @@ constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
 constexpr int kMaxPerLane = 32;  // C <= 1024
 
-// Order: larger score first; equal scores: lower candidate index first.
+// Order: larger score first; equal scores (-0.0 == +0.0): lower candidate index first.  NaN is not a
+// candidate: it is marked taken when loaded, so `better` only ever compares numbers (the order of
+// ncf_topk_rows).  A NaN in the order would break it: every comparison with NaN is false.
 __device__ __forceinline__ bool better(float v, int i, float bv, int bi) {
   return (v > bv) || (v == bv && i < bi);
 }
@@ -35,7 +37,7 @@ __global__ void __launch_bounds__(kThreads) eval_rank_kernel(const float* __rest
     for (int q = 0; q < kMaxPerLane; ++q) {
       const int c = lane + 32 * q;
       v[q] = (q < nq && c < C) ? s[c] : 0.f;
-      if (c >= C) taken |= (1u << q);
+      if (c >= C || v[q] != v[q]) taken |= (1u << q);
     }
     int my_rank = -1;
     for (int j = 0; j < k; ++j) {
@@ -51,6 +53,11 @@ __global__ void __launch_bounds__(kThreads) eval_rank_kernel(const float* __rest
         const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
         if (oi != 0x7fffffff && (bi == 0x7fffffff || better(ov, oi, bv, bi))) { bv = ov; bi = oi; }
+      }
+      if (bi == 0x7fffffff) {  // fewer than k candidates in the row (warp-uniform): pad with -1
+        if (lane == 0 && topk_idx != nullptr)
+          for (int jj = j; jj < k; ++jj) topk_idx[u * k + jj] = -1;
+        break;
       }
       if ((bi & 31) == lane) taken |= 1u << (bi >> 5);
       if (bi == 0) my_rank = j;

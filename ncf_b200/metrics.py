@@ -6,6 +6,11 @@ one fused launch and ranks them with one warp per user (ncf_eval_users).  The he
 column 0 of each candidate row (reference src/data/datasets.py:31-34); ties go to the lower
 candidate index.  NDCG is derived from the device rank on the host as 1/np.log2(rank+2) in float64,
 which is the reference's own expression (metrics.py:22), so the returned lists compare equal.
+
+A NaN score is not a candidate, so a user whose held-out score is NaN is a miss (HR 0, NDCG 0).  A
+model that has diverged to NaN, or an id outside the tables (the forward gives NaN for it), scores
+HR = 0 rather than a perfect one.  This departs from the reference on purpose: its torch.topk ranks
+NaN above every number and counts a NaN held-out item as a hit.
 """
 from __future__ import annotations
 
