@@ -113,7 +113,8 @@ int ncf_version(void);
 const char* ncf_last_error(void);
 /* which tile-kernel family the calling thread's last forward / training call ran on:
  * 0 none yet, 1 generic (FMA), 2 mma.sync tensor path, 3 tcgen05/TMEM path, 4 thread-per-sample FMA kernel
- * for narrow towers (factor_num 8) (diagnostic; tests) */
+ * for narrow towers (factor_num 8), 5 layer-per-launch FMA forward for wide towers at batches up to 2048
+ * (forward only) (diagnostic; tests) */
 int ncf_last_tile_path(void);
 /* Measurement aid for bench.py: with profiling on, every training step on the tcgen05 path records
  * the CUDA-event time of each of its launches (and synchronises the stream).  ncf_profile_read

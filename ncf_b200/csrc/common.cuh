@@ -14,7 +14,9 @@ int check_cuda(cudaError_t e, const char* what);
 int num_sms();
 // records "embedding-row gradients complete" on `st` (see ncf_wait_embedding_grads)
 int mark_embedding_grads_done(cudaStream_t st);
-extern thread_local int g_tile_path;  // 1 generic, 2 mma.sync, 3 tcgen05 (ncf_last_tile_path)
+// ncf_last_tile_path: 1 generic, 2 mma.sync, 3 tcgen05, 4 thread-per-sample, 5 layer-per-launch forward; chosen
+// by ncf::tile_path (step.cu)
+extern thread_local int g_tile_path;
 
 #define NCF_REQUIRE(cond, ...)        \
   do {                                \

@@ -89,14 +89,10 @@ extern "C" int ncf_eval_rank(const float* scores, int64_t n, int32_t C, int32_t 
   return NCF_OK;
 }
 
-namespace ncf {
-int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t workspace_bytes,
-                     cudaStream_t st);
-}
-
 // workspace = [scores n*C floats (used only when scores_out is NULL)] [forward workspace]
 extern "C" int64_t ncf_eval_workspace_bytes(const NcfModel* m, int64_t n, int32_t C) {
   if (n < 0 || C < 1) return -1;
+  // user_div = 0 bounds the call's user_div = C: for C <= 1024 the tcgen05 sub-batch floor(262144 / C) * C <= 262144
   const int64_t fw = ncf_forward_workspace_bytes(m, n * C);
   if (fw < 0) return -1;
   return ncf::align_up(n * C * 4, 256) + fw + 256;

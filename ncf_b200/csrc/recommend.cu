@@ -233,11 +233,6 @@ int grid_for(int64_t n, int per_sm) {
 
 }  // namespace
 
-namespace ncf {
-int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t workspace_bytes, cudaStream_t st);
-int64_t forward_workspace_bytes(const TileParams& p);
-}  // namespace ncf
-
 extern "C" int ncf_mask_items(float* scores, int64_t n, int64_t C, const int64_t* users, int64_t user_num,
                               const int64_t* rowptr, const int32_t* col, void* stream) {
   NCF_REQUIRE(n >= 0, "ncf_mask_items: negative n");

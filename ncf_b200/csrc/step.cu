@@ -30,68 +30,73 @@ __global__ void loss_grad_kernel(const float* __restrict__ logits, const float* 
   }
 }
 
-int64_t scratch_floats(const NcfModel* m, int64_t B) {
-  if (m->model_type == NCF_GMF) return 0;
-  ncf::TowerShape ts = ncf::make_tower_shape(m->model_type, m->factor_num, m->num_layers);
-  int64_t n = 0;
-  for (int k = 1; k < ts.L; ++k) n += B * ts.width[k];   // act[k]
-  for (int k = 1; k <= ts.L; ++k) n += B * ts.width[k];  // delta[k]
-  return n;
+// tile_path below the thread-per-sample kernel.  The training query sizes for this path: the thread-per-sample
+// kernel needs no workspace, and the query then does not depend on the weight alignment that kernel checks.
+int tensor_path(const TileParams& p, bool train) {
+  if (ncf::umma_eligible(p)) return 3;
+  if (!train && ncf::wide_eligible(p)) return 5;
+  return ncf::mma_tile_rows(p) != 0 ? 2 : 1;
+}
+
+int64_t train_workspace_bytes(const TileParams& p) {
+  return ncf::align_up(ncf::tile_workspace_floats(tensor_path(p, true), p, p.B, true) * 4, 256) + 256;
+}
+
+// The one workspace rule of the forward and training entry points: a call that needs `need` > 0 bytes gets a
+// non-NULL workspace of at least that size.
+int check_workspace(const char* who, const void* workspace, int64_t workspace_bytes, int64_t need) {
+  if (need > 0 && (!workspace || workspace_bytes < need)) {
+    ncf::set_error("%s: workspace too small (%lld < %lld)", who, (long long)workspace_bytes, (long long)need);
+    return NCF_ERR_WORKSPACE;
+  }
+  return NCF_OK;
 }
 
 }  // namespace
 
 namespace ncf {
 
-// Forward over p.B samples on whichever tile kernel the shape is eligible for.  The tensor-pipe
-// path needs mma_split_floats(p) floats of workspace for the pre-split weights.
-int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t workspace_bytes,
-                     cudaStream_t st) {
-  if (small_eligible(p)) {
-    g_tile_path = 4;
-    return launch_small_forward(p, st);
+int tile_path(const TileParams& p, bool train) { return small_eligible(p) ? 4 : tensor_path(p, train); }
+
+int64_t tile_workspace_floats(int path, const TileParams& p, int64_t B, bool train) {
+  switch (path) {
+    case 1: return train ? scratch_floats(p, B, true) : 0;  // the generic forward keeps its rows on chip
+    case 2: return image_floats(p);
+    // + 64: the scratch starts at the next 256-byte boundary after the images
+    case 3: return image_floats(p) + scratch_floats(p, train ? B : std::min(B, forward_sub(p)), train) + 64;
+    case 5: return wide_workspace_floats(p, B);
+    default: return 0;
   }
-  if (umma_eligible(p)) {
-    const int64_t need = umma_forward_workspace_floats(p, p.B) * 4;
-    if (!workspace || workspace_bytes < need) {
-      set_error("forward: workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
-      return NCF_ERR_WORKSPACE;
-    }
-    g_tile_path = 3;
-    return launch_umma_forward(p, tower_passes(m), (float*)workspace, st);
-  }
-  if (wide_eligible(p)) {
-    const int64_t need = wide_workspace_floats(p, p.B) * 4;
-    if (!workspace || workspace_bytes < need) {
-      set_error("forward: workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
-      return NCF_ERR_WORKSPACE;
-    }
-    g_tile_path = 5;
-    return launch_wide_forward(p, (float*)workspace, st);
-  }
-  g_tile_path = mma_tile_rows(p) == 0 ? 1 : 2;
-  if (mma_tile_rows(p) == 0) return launch_generic_forward(p, st);
-  const int64_t need = mma_split_floats(p) * 4;
-  if (!workspace || workspace_bytes < need) {
-    set_error("forward: workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
-    return NCF_ERR_WORKSPACE;
-  }
-  int rc = mma_prepare_weights(p, (float*)workspace, st);
-  if (rc != NCF_OK) return rc;
-  return launch_mma_forward(p, tower_passes(m), st);
 }
 
-// Workspace of forward_dispatch for any batch up to p.B (with p.user_div as the caller will pass it).
+int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t workspace_bytes,
+                     cudaStream_t st) {
+  const int path = tile_path(p, false);
+  int rc = check_workspace("forward", workspace, workspace_bytes, tile_workspace_floats(path, p, p.B, false) * 4);
+  if (rc != NCF_OK) return rc;
+  g_tile_path = path;
+  float* ws = (float*)workspace;
+  switch (path) {
+    case 4: return launch_small_forward(p, st);
+    case 3: return launch_umma_forward(p, tower_passes(m), ws, st);
+    case 5: return launch_wide_forward(p, ws, st);
+    case 2:
+      rc = mma_prepare_weights(p, ws, st);
+      return rc != NCF_OK ? rc : launch_mma_forward(p, mma_tile_rows(p), tower_passes(m), st);
+    default: return launch_generic_forward(p, st);
+  }
+}
+
+// The most any batch up to p.B can need: each path that consumes workspace, at the largest batch its own rule
+// admits (the order of tile_path is not applied, so the value is an upper bound).
 int64_t forward_workspace_bytes(const TileParams& p) {
-  const int64_t B = p.B;
-  int64_t bytes = mma_tile_rows(p) ? align_up(mma_split_floats(p) * 4, 256) : 0;
+  int64_t bytes = 0;
+  if (mma_tile_rows(p)) bytes = align_up(tile_workspace_floats(2, p, p.B, false) * 4, 256);
   if (umma_eligible(p))
-    bytes = std::max(bytes, align_up(umma_forward_workspace_floats(p, B) * 4, 256) + 256);
-  // any batch up to B may be passed with a workspace of this size: cover the small-batch path as well
+    bytes = std::max(bytes, align_up(tile_workspace_floats(3, p, p.B, false) * 4, 256) + 256);
   TileParams ps = p;
-  ps.B = std::min<int64_t>(B, 2048);
-  if (ps.B > 0 && wide_eligible(ps))
-    bytes = std::max(bytes, align_up(wide_workspace_floats(ps, ps.B) * 4, 256));
+  ps.B = std::min(p.B, kWideMaxB);
+  if (wide_eligible(ps)) bytes = std::max(bytes, align_up(tile_workspace_floats(5, ps, ps.B, false) * 4, 256));
   return bytes;
 }
 
@@ -140,9 +145,7 @@ extern "C" int64_t ncf_train_workspace_bytes(const NcfModel* m, int64_t B) {
   TileParams p{};
   ncf::fill_model_params(p, m);
   p.B = B;
-  int64_t floats = ncf::mma_tile_rows(p) ? ncf::mma_split_floats(p) : scratch_floats(m, B);
-  if (ncf::umma_eligible(p)) floats = std::max(floats, ncf::umma_train_workspace_floats(p, B));
-  return ncf::align_up(floats * 4, 256) + 256;
+  return train_workspace_bytes(p);
 }
 
 static int train_common(const NcfModel* m, const NcfGrads* g, const int64_t* user,
@@ -196,12 +199,6 @@ static int train_common(const NcfModel* m, const NcfGrads* g, const int64_t* use
     NCF_REQUIRE(g->g_user_gmf && g->g_item_gmf, "ncf_train_step_grads: GMF grad buffers are NULL");
   if (m->model_type != NCF_GMF)
     NCF_REQUIRE(g->g_user_mlp && g->g_item_mlp, "ncf_train_step_grads: MLP grad buffers are NULL");
-  const int64_t need = ncf_train_workspace_bytes(m, B);
-  if (workspace_bytes < need || (need > 256 && !workspace)) {
-    ncf::set_error("ncf_train_step_grads: workspace too small (%lld < %lld)",
-                   (long long)workspace_bytes, (long long)need);
-    return NCF_ERR_WORKSPACE;
-  }
   TileParams p{};
   ncf::fill_model_params(p, m);
   ncf::fill_grad_params(p, g);
@@ -215,30 +212,23 @@ static int train_common(const NcfModel* m, const NcfGrads* g, const int64_t* use
   p.invB = 1.f / (float)(B_norm > 0 ? B_norm : B);  // mean over the (global) batch
   p.logits = logits_out;
   p.loss_accum = loss_accum;
-  if (ncf::small_eligible(p)) {
-    ncf::g_tile_path = 4;
-    rc = ncf::launch_small_train(p, (cudaStream_t)stream);
-    if (rc != NCF_OK) return rc;
-    return ncf::mark_embedding_grads_done((cudaStream_t)stream);
-  }
-  if (ncf::umma_eligible(p)) {
-    ncf::g_tile_path = 3;
-    return ncf::launch_umma_train(p, ncf::tower_passes(m), (float*)workspace, (cudaStream_t)stream);
-  }
-  ncf::g_tile_path = ncf::mma_tile_rows(p) != 0 ? 2 : 1;
-  if (ncf::mma_tile_rows(p) != 0) {
-    rc = ncf::mma_prepare_weights(p, (float*)workspace, (cudaStream_t)stream);
-    if (rc != NCF_OK) return rc;
-    rc = ncf::launch_mma_train(p, ncf::tower_passes(m), (cudaStream_t)stream);
-    if (rc != NCF_OK) return rc;
-    return ncf::mark_embedding_grads_done((cudaStream_t)stream);
-  }
-  if (m->model_type != NCF_GMF) {
-    float* ws = (float*)workspace;
-    for (int k = 1; k < p.L; ++k) { p.act[k] = ws; ws += B * p.W[k]; }
-    for (int k = 1; k <= p.L; ++k) { p.delta[k] = ws; ws += B * p.W[k]; }
-  }
-  rc = ncf::launch_generic_train(p, (cudaStream_t)stream);
+  const int path = ncf::tile_path(p, true);
+  rc = check_workspace("ncf_train_step_grads", workspace, workspace_bytes, train_workspace_bytes(p));
   if (rc != NCF_OK) return rc;
-  return ncf::mark_embedding_grads_done((cudaStream_t)stream);
+  ncf::g_tile_path = path;
+  float* ws = (float*)workspace;
+  const cudaStream_t st = (cudaStream_t)stream;
+  switch (path) {
+    case 4: rc = ncf::launch_small_train(p, st); break;
+    case 3: return ncf::launch_umma_train(p, ncf::tower_passes(m), ws, st);  // marks the embedding grads itself
+    case 2:
+      rc = ncf::mma_prepare_weights(p, ws, st);
+      if (rc == NCF_OK) rc = ncf::launch_mma_train(p, ncf::mma_tile_rows(p), ncf::tower_passes(m), st);
+      break;
+    default:
+      ncf::carve_scratch(p, ws, B, true);
+      rc = ncf::launch_generic_train(p, st);
+  }
+  if (rc != NCF_OK) return rc;
+  return ncf::mark_embedding_grads_done(st);
 }

@@ -658,39 +658,22 @@ int mma_tile_rows(const TileParams& p_in) {
   return 0;
 }
 
-int64_t mma_split_floats(const TileParams& p) {
-  int64_t n = 0;
-  for (int k = 0; k < p.L; ++k) n += 2 * 2 * (int64_t)p.W[k] * p.W[k + 1];
-  return n;
-}
-
-// ws: mma_split_floats(p) floats.  Fills p.wsplit_f / p.wsplit_b and launches the split.
+// ws: image_floats(p) floats.  Points p.wsplit_f / p.wsplit_b into it and launches the split.
 int mma_prepare_weights(TileParams& p, float* ws, cudaStream_t st) {
-  for (int k = 0; k < p.L; ++k) {
-    const int64_t n = 2 * (int64_t)p.W[k] * p.W[k + 1];
-    p.wsplit_f[k] = ws;
-    p.wsplit_b[k] = ws + n;
-    ws += 2 * n;
-  }
+  point_images(p, ws);
   split_weights_kernel<<<dim3(32, p.L), 256, 0, st>>>(p);
   NCF_LAUNCH_CHECK("split_weights_kernel");
   return NCF_OK;
 }
 
-int launch_mma_forward(TileParams& p, int passes, cudaStream_t st) {
-  const int tm = mma_tile_rows(p);
-  if (tm == 64) return passes == 3 ? launch_mma<3, 64, false>(p, st) : launch_mma<1, 64, false>(p, st);
-  if (tm == 32) return passes == 3 ? launch_mma<3, 32, false>(p, st) : launch_mma<1, 32, false>(p, st);
-  set_error("model not eligible for the mma tile kernel");
-  return NCF_ERR_ARG;
+int launch_mma_forward(TileParams& p, int tile_rows, int passes, cudaStream_t st) {
+  if (tile_rows == 64) return passes == 3 ? launch_mma<3, 64, false>(p, st) : launch_mma<1, 64, false>(p, st);
+  return passes == 3 ? launch_mma<3, 32, false>(p, st) : launch_mma<1, 32, false>(p, st);
 }
 
-int launch_mma_train(TileParams& p, int passes, cudaStream_t st) {
-  const int tm = mma_tile_rows(p);
-  if (tm == 64) return passes == 3 ? launch_mma<3, 64, true>(p, st) : launch_mma<1, 64, true>(p, st);
-  if (tm == 32) return passes == 3 ? launch_mma<3, 32, true>(p, st) : launch_mma<1, 32, true>(p, st);
-  set_error("model not eligible for the mma tile kernel");
-  return NCF_ERR_ARG;
+int launch_mma_train(TileParams& p, int tile_rows, int passes, cudaStream_t st) {
+  if (tile_rows == 64) return passes == 3 ? launch_mma<3, 64, true>(p, st) : launch_mma<1, 64, true>(p, st);
+  return passes == 3 ? launch_mma<3, 32, true>(p, st) : launch_mma<1, 32, true>(p, st);
 }
 
 }  // namespace ncf

@@ -27,10 +27,11 @@ struct TileParams {
   int32_t *uflag, *iflag, *tcount;
   int64_t *ulist, *ilist;
   int64_t w_off[NCF_MAX_LAYERS], b_off[NCF_MAX_LAYERS], pw_off, pb_off;
-  // HBM scratch of per-sample activations / deltas (generic path)
+  // HBM scratch of per-sample activations / deltas (generic training, tcgen05), laid out by carve_scratch
   float* act[NCF_MAX_LAYERS + 1];    // act[k],   k = 1..L-1 : [B, W[k]]
   float* delta[NCF_MAX_LAYERS + 1];  // delta[k], k = 1..L   : [B, W[k]]
-  // pre-split (hi, lo) TF32 weights for the mma path: forward operand and transposed operand
+  // (hi, lo) weight images of the mma.sync and tcgen05 paths, forward operand and transposed operand, laid out
+  // by point_images
   float* wsplit_f[NCF_MAX_LAYERS];
   float* wsplit_b[NCF_MAX_LAYERS];
   // shared-memory layout (float offsets), filled by the launcher
@@ -79,15 +80,59 @@ inline void fill_grad_params(TileParams& p, const NcfGrads* g) {
   p.tcount = g->touched_count;
 }
 
+// Workspace layouts shared by the tile paths.  Weight images: per layer k, 2 * W[k] * W[k+1] floats of
+// forward operand, then as many of transposed operand.
+inline int64_t image_floats(const TileParams& p) {
+  int64_t n = 0;
+  for (int k = 0; k < p.L; ++k) n += 2 * 2 * (int64_t)p.W[k] * p.W[k + 1];
+  return n;
+}
+// points wsplit_f / wsplit_b into ws; returns the end of the images
+inline float* point_images(TileParams& p, float* ws) {
+  for (int k = 0; k < p.L; ++k) {
+    const int64_t n = 2 * (int64_t)p.W[k] * p.W[k + 1];
+    p.wsplit_f[k] = ws;
+    p.wsplit_b[k] = ws + n;
+    ws += 2 * n;
+  }
+  return ws;
+}
+// act[1..L-1] and, when training, delta[1..L] for B samples; GMF has no tower and no scratch
+inline int64_t scratch_floats(const TileParams& p, int64_t B, bool train) {
+  if (p.type == NCF_GMF) return 0;
+  int64_t n = 0;
+  for (int k = 1; k < p.L; ++k) n += B * p.W[k];
+  if (train)
+    for (int k = 1; k <= p.L; ++k) n += B * p.W[k];
+  return n;
+}
+inline void carve_scratch(TileParams& p, float* ws, int64_t B, bool train) {
+  if (p.type == NCF_GMF) return;
+  for (int k = 1; k < p.L; ++k) { p.act[k] = ws; ws += B * p.W[k]; }
+  if (train)
+    for (int k = 1; k <= p.L; ++k) { p.delta[k] = ws; ws += B * p.W[k]; }
+}
+
+// The tile path of a forward (train = false) or training call, as ncf_last_tile_path() reports it: 4 the
+// thread-per-sample kernel, 3 tcgen05, 5 the layer-per-launch forward (inference only), 2 mma.sync, 1 generic;
+// the first in that order whose eligibility rule below admits p.  step.cu holds this order and nothing else
+// restates it: the launchers and the workspace queries go through tile_path / tile_workspace_floats.
+int tile_path(const TileParams& p, bool train);
+// floats of workspace that `path` consumes for a call over B samples
+int64_t tile_workspace_floats(int path, const TileParams& p, int64_t B, bool train);
+// forward over p.B samples on tile_path(p, false), with the workspace checked against its need
+int forward_dispatch(TileParams& p, const NcfModel* m, void* workspace, int64_t workspace_bytes, cudaStream_t st);
+// workspace that serves forward_dispatch for every batch up to p.B (with p.user_div as the caller will pass it)
+int64_t forward_workspace_bytes(const TileParams& p);
+
 int launch_generic_forward(TileParams& p, cudaStream_t st);
 int launch_generic_train(TileParams& p, cudaStream_t st);
 
-// tensor-pipe path (tile_mma.cu): eligible when mma_tile_rows(p) != 0
+// tensor-pipe path (tile_mma.cu): eligible when mma_tile_rows(p) != 0, the tile height (32 or 64)
 int mma_tile_rows(const TileParams& p);
-int64_t mma_split_floats(const TileParams& p);
 int mma_prepare_weights(TileParams& p, float* ws, cudaStream_t st);
-int launch_mma_forward(TileParams& p, int passes, cudaStream_t st);
-int launch_mma_train(TileParams& p, int passes, cudaStream_t st);
+int launch_mma_forward(TileParams& p, int tile_rows, int passes, cudaStream_t st);
+int launch_mma_train(TileParams& p, int tile_rows, int passes, cudaStream_t st);
 inline int tower_passes(const NcfModel* m) { return m->tower_math == NCF_MATH_TF32 ? 1 : 3; }
 
 // narrow towers, one thread per sample on the FMA pipe (tile_small.cu): factor_num 8, 1..3 layers
@@ -96,14 +141,14 @@ int launch_small_forward(TileParams& p, cudaStream_t st);
 int launch_small_train(TileParams& p, cudaStream_t st);
 
 // wide towers at small batches, forward only: one launch per layer over many CTAs (tile_wide.cu)
+constexpr int64_t kWideMaxB = 2048;       // largest batch it takes
 bool wide_eligible(const TileParams& p);  // reads p.B
 int64_t wide_workspace_floats(const TileParams& p, int64_t B);
 int launch_wide_forward(TileParams& p, float* ws, cudaStream_t st);
 
 // tcgen05 path (tile_umma.cu): large batches, tower widths that are power-of-two multiples of 32
 bool umma_eligible(const TileParams& p);  // reads p.B
-int64_t umma_forward_workspace_floats(const TileParams& p, int64_t B);
-int64_t umma_train_workspace_floats(const TileParams& p, int64_t B);
+int64_t forward_sub(const TileParams& p);  // rows of one inference sub-batch
 int launch_umma_forward(TileParams& p, int passes, float* ws, cudaStream_t st);
 int launch_umma_train(TileParams& p, int passes, float* ws, cudaStream_t st);
 

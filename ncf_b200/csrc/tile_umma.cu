@@ -1616,61 +1616,31 @@ bool umma_eligible(const TileParams& p) {
   return blocks <= 12;
 }
 
-int64_t umma_image_floats(const TileParams& p) {
-  int64_t n = 0;
-  for (int k = 0; k < p.L; ++k) n += 2 * 2 * (int64_t)p.W[k] * p.W[k + 1];
-  return n;
-}
-
-int64_t umma_scratch_floats(const TileParams& p, int64_t B, bool train) {
-  int64_t n = 0;
-  for (int k = 1; k < p.L; ++k) n += B * p.W[k];
-  if (train)
-    for (int k = 1; k <= p.L; ++k) n += B * p.W[k];
-  return n;
-}
-
 constexpr int64_t kForwardSub = 262144;  // inference sub-batch: bounds the activation scratch
 
-// rows of one inference sub-batch: a whole number of users when one user covers user_div rows
-static int64_t forward_sub(const TileParams& p) {
+// a whole number of users when one user covers user_div rows
+int64_t forward_sub(const TileParams& p) {
   return p.user_div > 0 ? std::max<int64_t>(1, kForwardSub / p.user_div) * p.user_div : kForwardSub;
 }
 
-int64_t umma_forward_workspace_floats(const TileParams& p, int64_t B) {
-  return umma_image_floats(p) + umma_scratch_floats(p, std::min<int64_t>(B, forward_sub(p)), false) + 64;
-}
-int64_t umma_train_workspace_floats(const TileParams& p, int64_t B) {
-  return umma_image_floats(p) + umma_scratch_floats(p, B, true) + 64;
-}
-
-static float* carve(TileParams& p, float* ws, int64_t B, bool train, cudaStream_t st, int* rc) {
-  for (int k = 0; k < p.L; ++k) {
-    const int64_t n = 2 * (int64_t)p.W[k] * p.W[k + 1];
-    p.wsplit_f[k] = ws;
-    p.wsplit_b[k] = ws + n;
-    ws += 2 * n;
-  }
-  ws = (float*)(((uintptr_t)ws + 255) & ~(uintptr_t)255);
-  for (int k = 1; k < p.L; ++k) { p.act[k] = ws; ws += B * p.W[k]; }
-  if (train)
-    for (int k = 1; k <= p.L; ++k) { p.delta[k] = ws; ws += B * p.W[k]; }
+// ws: tile_workspace_floats(3, p, B, train) floats.  Images, then the scratch of B rows from the next 256-byte
+// boundary; launches the image kernel.
+static int carve(TileParams& p, float* ws, int64_t B, bool train, cudaStream_t st) {
+  ws = point_images(p, ws);
+  carve_scratch(p, (float*)(((uintptr_t)ws + 255) & ~(uintptr_t)255), B, train);
   umma_weight_images_kernel<<<dim3(64, 2 * p.L), 256, 0, st>>>(p);
-  *rc = check_cuda(cudaGetLastError(), "umma_weight_images_kernel");
-  return ws;
+  return check_cuda(cudaGetLastError(), "umma_weight_images_kernel");
 }
 
 int launch_umma_forward(TileParams& p, int passes, float* ws, cudaStream_t st) {
   int rc;
   const int64_t B = p.B;
   if (tower_fused_ok(p)) {
-    carve(p, ws, 0, false, st, &rc);
-    if (rc != NCF_OK) return rc;
+    if ((rc = carve(p, ws, 0, false, st)) != NCF_OK) return rc;
     return launch_tower<false>(p, passes, st);
   }
   const int64_t sub = forward_sub(p);
-  carve(p, ws, std::min(B, sub), false, st, &rc);
-  if (rc != NCF_OK) return rc;
+  if ((rc = carve(p, ws, std::min(B, sub), false, st)) != NCF_OK) return rc;
   const int64_t* user = p.user;
   const int64_t* item = p.item;
   float* logits = p.logits;
@@ -1688,8 +1658,7 @@ int launch_umma_forward(TileParams& p, int passes, float* ws, cudaStream_t st) {
 int launch_umma_train(TileParams& p, int passes, float* ws, cudaStream_t st) {
   int rc;
   StepTimer timer(st);
-  carve(p, ws, p.B, true, st, &rc);
-  if (rc != NCF_OK) return rc;
+  if ((rc = carve(p, ws, p.B, true, st)) != NCF_OK) return rc;
   timer.mark("images");
   if (tower_fused_ok(p)) {
     rc = launch_tower<true>(p, passes, st);

@@ -19,7 +19,6 @@ namespace {
 
 constexpr int kT = 32;          // output tile: 32 samples x 32 outputs, K walked in chunks of 32
 constexpr int kWideThreads = 256;
-constexpr int64_t kWideMaxB = 2048;
 
 struct WideLayer {
   const float* in;       // [B, K] activations (layers > 0)
