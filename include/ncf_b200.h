@@ -275,12 +275,14 @@ int ncf_mark_rows(const NcfModel* m_host, const NcfGrads* g_host, const int64_t*
  * tables register a rank's own users and the item rows other ranks requested separately. */
 int ncf_mark_rows_side(const NcfModel* m_host, const NcfGrads* g_host, const int64_t* rows, int64_t n,
                        int32_t side, void* stream);
-/* Replays the pending zero-gradient Adam steps of every row currently in g's touched lists. */
+/* Replays the pending zero-gradient Adam steps of every row currently in g's touched lists.
+ * Bad hyper-parameters (outside 0 < beta1 < 1, 0 < beta2 < 1, eps > 0): NCF_ERR_ARG, nothing launched. */
 int ncf_adam_catchup(const NcfModel* m_host, const NcfGrads* g_host, const NcfAdamState* s_host,
                      NcfAdamHyper h, void* stream);
 /* ncf_adam_prepare: call BEFORE ncf_train_step_grads of the same batch.  Registers the batch's
  * distinct rows in g's touched lists and replays their pending zero-gradient steps, so that the
- * forward reads the rows exactly as the reference's dense Adam would have left them. */
+ * forward reads the rows exactly as the reference's dense Adam would have left them.  Bad hyper-parameters:
+ * NCF_ERR_ARG, nothing launched. */
 int ncf_adam_prepare(const NcfModel* m_host, const NcfGrads* g_host, const NcfAdamState* s_host,
                      NcfAdamHyper h, const int64_t* user, const int64_t* item, int64_t B,
                      void* stream);
@@ -339,6 +341,7 @@ int ncf_peer_free(void* dev_ptr);
 int ncf_ipc_export(const void* dev_ptr, void* handle64);
 int ncf_ipc_open(const void* handle64, void** dev_ptr_out);
 int ncf_ipc_close(void* dev_ptr);
+/* ncf_adam_flush (see above); bad hyper-parameters: NCF_ERR_ARG, nothing launched. */
 int ncf_adam_flush(const NcfModel* m_host, const NcfAdamState* s_host, NcfAdamHyper h,
                    void* stream);
 int ncf_sgd_step(const NcfModel* m_host, const NcfGrads* g_host, float lr, void* stream);

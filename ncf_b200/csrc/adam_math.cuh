@@ -1,5 +1,4 @@
-// Adam arithmetic shared by the optimiser kernels (optim.cu) and by tile kernels that replay pending
-// zero-gradient steps while they gather (tile_small.cu).  torch.optim.Adam single-tensor math (torch 2.11
+// Adam arithmetic of the optimiser kernels (optim.cu).  torch.optim.Adam single-tensor math (torch 2.11
 // optim/adam.py), per step t = 1, 2, ...:
 //   m <- m + (1-b1)(g - m);  v <- b2 v + (1-b2) g^2
 //   p <- p - (lr / (1-b1^t)) * m / (sqrt(v)/sqrt(1-b2^t) + eps)

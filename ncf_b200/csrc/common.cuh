@@ -82,6 +82,14 @@ __device__ __forceinline__ float4 ldg4(const float* p) {
   return __ldg(reinterpret_cast<const float4*>(p));
 }
 
+// Registers `row` in a touched list (the dedup the optimisers walk): the one thread that flips flag[row] from 0
+// appends the row to `list`, whose length is *count.  Returns whether this thread won.
+__device__ __forceinline__ bool claim_row(int32_t* flag, int64_t* list, int32_t* count, int64_t row) {
+  if (atomicExch(&flag[row], 1) != 0) return false;
+  list[atomicAdd(count, 1)] = row;
+  return true;
+}
+
 // The per-sample training objective, defined once for every tile kernel and loss_grad_kernel (the KD
 // objective of distill.cu is a different one): BCE-with-logits of logit x against label y, mixed with
 // the squared distance to the teacher logit t when there is a teacher (alpha weights the BCE term).

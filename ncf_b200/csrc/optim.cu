@@ -72,6 +72,69 @@ struct RowsParams {
   AdamConst c;
 };
 
+// ---- the touched-row protocol (DESIGN §3.2); last[side][r]: the step after which row r is current (0: never) ----
+// The zero-gradient steps last+1 .. now a row owes, now = *step (the last step taken).  kStep (a real step
+// follows): none for a row never stepped.  Replay only: false (nothing to do) for a row never stepped or current.
+template <bool kStep>
+__device__ __forceinline__ bool pending_gap(int32_t last, int64_t now, int& gap) {
+  if (kStep) {
+    gap = (last > 0) ? (int)(now - last) : 0;
+    return true;
+  }
+  gap = (int)(now - last);
+  return last > 0 && last < now;
+}
+
+// The warp's bias terms of steps last+1 .. last+min(gap, kMaxReplay) for replay_zero_steps_n; the first
+// __syncwarp keeps these writes behind the lanes still reading the previous row's terms.
+__device__ __forceinline__ void fill_bias_table(float* c1s, float* c2s, int32_t last, int gap, const AdamConst& c,
+                                                int lane) {
+  __syncwarp();
+  for (int j = lane; j < min(gap, kMaxReplay); j += 32) {
+    const float s = (float)(last + 1 + j);
+    c1s[j] = bias_c1(c, s);
+    c2s[j] = bias_c2(c, s);
+  }
+  __syncwarp();
+}
+
+// Entry e of the rows a kernel walks, n0 users then the items: its side, and its row in the touched list or
+// in the row range [row0, row0 + rows) of the all-rows modes.
+__device__ __forceinline__ int entry_side(int64_t e, int64_t n0) { return e < n0 ? 0 : 1; }
+template <bool kList>
+__device__ __forceinline__ int64_t entry_row(const RowsParams& q, int64_t e, int64_t n0, int side) {
+  return kList ? q.list[side][side ? e - n0 : e] : q.row0[side] + (side ? e - n0 : e);
+}
+
+// the row is current at step t; a real step also takes it out of the touched set
+template <bool kStep>
+__device__ __forceinline__ void stamp_row(const RowsParams& q, int side, int64_t r, int64_t t, int lane) {
+  if (lane == 0) {
+    q.last[side][r] = (int32_t)t;
+    if (kStep) q.flag[side][r] = 0;
+  }
+}
+
+// Row r of the GMF and then the MLP table: the gap's replay, (kStep) the real step t consuming the gradient,
+// the stamp.
+template <bool kStep>
+__device__ __forceinline__ void update_row(const RowsParams& q, int side, int64_t r, int gap, bool vec, const float* c1s,
+                                           const float* c2s, int64_t t, float c1t, float c2t, int lane) {
+  if (q.has_gmf) {
+    const int64_t o = r * q.f;
+    float* G = kStep ? q.g_gmf[side] + o : nullptr;
+    if (vec) adam_row<4>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, G, q.f, gap, c1s, c2s, c1t, c2t, q.c, lane);
+    else adam_row<1>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, G, q.f, gap, c1s, c2s, c1t, c2t, q.c, lane);
+  }
+  if (q.has_mlp) {
+    const int64_t o = r * q.d;
+    float* G = kStep ? q.g_mlp[side] + o : nullptr;
+    if (vec) adam_row<4>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, G, q.d, gap, c1s, c2s, c1t, c2t, q.c, lane);
+    else adam_row<1>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, G, q.d, gap, c1s, c2s, c1t, c2t, q.c, lane);
+  }
+  stamp_row<kStep>(q, side, r, t, lane);
+}
+
 struct DenseSeg {
   float* p;
   int64_t off, n;
@@ -133,17 +196,6 @@ __global__ void step_tail_kernel(const StepTail tail) { step_tail(tail, *tail.st
 // mode 3: Adam step on ALL rows (the reference's dense optimiser as it is): when a step touches a
 // large share of the tables, streaming every row once is cheaper than list + catch-up + row gather.
 template <int MODE>
-__device__ __forceinline__ void adam_rows_body(const RowsParams& q, int64_t step_now);
-
-// mode 0 ends the step (step_tail); the other modes ignore `tail`
-template <int MODE>
-__global__ void __launch_bounds__(kThreads) adam_rows_kernel(const RowsParams q, const StepTail tail) {
-  const int64_t step_now = *q.step;
-  adam_rows_body<MODE>(q, step_now);
-  if (MODE == 0) step_tail(tail, step_now);
-}
-
-template <int MODE>
 __device__ __forceinline__ void adam_rows_body(const RowsParams& q, const int64_t step_now) {
   __shared__ float c1_sm[kWarps][kMaxReplay];
   __shared__ float c2_sm[kWarps][kMaxReplay];
@@ -165,11 +217,11 @@ __device__ __forceinline__ void adam_rows_body(const RowsParams& q, const int64_
   if (vec && q.has_gmf && q.has_mlp && q.f <= 128 && q.d <= 128) {
     const bool lg = lane * 4 < q.f, lm = lane * 4 < q.d;
     auto fetch = [&](int64_t e, int& side, int64_t& r, int32_t& last) {
-      side = e < n0 ? 0 : 1;
+      side = entry_side(e, n0);
       r = 0;
       last = 0;
       if (e < total) {
-        r = kList ? q.list[side][side ? e - n0 : e] : q.row0[side] + (side ? e - n0 : e);
+        r = entry_row<kList>(q, e, n0, side);
         last = q.last[side][r];
       }
     };
@@ -180,12 +232,7 @@ __device__ __forceinline__ void adam_rows_body(const RowsParams& q, const int64_
     for (int64_t e = wid; e < total; e += nw, side = nside, r = nr, last = nlast) {
       fetch(e + nw, nside, nr, nlast);
       int gap;
-      if (kStep) {
-        gap = (last > 0) ? (int)(t - 1 - last) : 0;
-      } else {
-        if (last <= 0 || last >= t) continue;
-        gap = (int)(t - last);
-      }
+      if (!pending_gap<kStep>(last, step_now, gap)) continue;
       const int64_t og = r * q.f + lane * 4, om = r * q.d + lane * 4;
       float4 pg = make_float4(0, 0, 0, 0), mg = pg, vg = pg, gg = pg, pm = pg, mm = pg, vm = pg, gm = pg;
       if (lg) {
@@ -200,14 +247,7 @@ __device__ __forceinline__ void adam_rows_body(const RowsParams& q, const int64_
         vm = *reinterpret_cast<const float4*>(q.v_mlp[side] + om);
         if (kStep) gm = *reinterpret_cast<const float4*>(q.g_mlp[side] + om);
       }
-      __syncwarp();
-      const int n = min(gap, kMaxReplay);
-      for (int j = lane; j < n; j += 32) {
-        const float s = (float)(last + 1 + j);
-        c1s[j] = bias_c1(q.c, s);
-        c2s[j] = bias_c2(q.c, s);
-      }
-      __syncwarp();
+      fill_bias_table(c1s, c2s, last, gap, q.c, lane);
       // the lane's eight elements (4 of the GMF row, 4 of the MLP row) replay together
       float pe[8] = {pg.x, pg.y, pg.z, pg.w, pm.x, pm.y, pm.z, pm.w};
       float me[8] = {mg.x, mg.y, mg.z, mg.w, mm.x, mm.y, mm.z, mm.w};
@@ -233,49 +273,27 @@ __device__ __forceinline__ void adam_rows_body(const RowsParams& q, const int64_
         *reinterpret_cast<float4*>(q.v_mlp[side] + om) = vm;
         if (kStep) *reinterpret_cast<float4*>(q.g_mlp[side] + om) = make_float4(0, 0, 0, 0);
       }
-      if (lane == 0) {
-        q.last[side][r] = (int32_t)t;
-        if (kStep) q.flag[side][r] = 0;
-      }
+      stamp_row<kStep>(q, side, r, t, lane);
     }
     return;
   }
   for (int64_t e = wid; e < total; e += nw) {
-    const int side = e < n0 ? 0 : 1;
-    const int64_t r = kList ? q.list[side][side ? e - n0 : e] : q.row0[side] + (side ? e - n0 : e);
+    const int side = entry_side(e, n0);
+    const int64_t r = entry_row<kList>(q, e, n0, side);
     const int32_t last = q.last[side][r];
     int gap;
-    if (kStep) {
-      gap = (last > 0) ? (int)(t - 1 - last) : 0;
-    } else {
-      if (last <= 0 || last >= t) continue;
-      gap = (int)(t - last);
-    }
-    __syncwarp();
-    const int n = min(gap, kMaxReplay);
-    for (int j = lane; j < n; j += 32) {
-      const float s = (float)(last + 1 + j);
-      c1s[j] = bias_c1(q.c, s);
-      c2s[j] = bias_c2(q.c, s);
-    }
-    __syncwarp();
-    if (q.has_gmf) {
-      const int64_t o = r * q.f;
-      float* G = kStep ? q.g_gmf[side] + o : nullptr;
-      if (vec) adam_row<4>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, G, q.f, gap, c1s, c2s, c1t, c2t, q.c, lane);
-      else adam_row<1>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, G, q.f, gap, c1s, c2s, c1t, c2t, q.c, lane);
-    }
-    if (q.has_mlp) {
-      const int64_t o = r * q.d;
-      float* G = kStep ? q.g_mlp[side] + o : nullptr;
-      if (vec) adam_row<4>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, G, q.d, gap, c1s, c2s, c1t, c2t, q.c, lane);
-      else adam_row<1>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, G, q.d, gap, c1s, c2s, c1t, c2t, q.c, lane);
-    }
-    if (lane == 0) {
-      q.last[side][r] = (int32_t)t;
-      if (kStep) q.flag[side][r] = 0;
-    }
+    if (!pending_gap<kStep>(last, step_now, gap)) continue;
+    fill_bias_table(c1s, c2s, last, gap, q.c, lane);
+    update_row<kStep>(q, side, r, gap, vec, c1s, c2s, t, c1t, c2t, lane);
   }
+}
+
+// mode 0 ends the step (step_tail); the other modes ignore `tail`
+template <int MODE>
+__global__ void __launch_bounds__(kThreads) adam_rows_kernel(const RowsParams q, const StepTail tail) {
+  const int64_t step_now = *q.step;
+  adam_rows_body<MODE>(q, step_now);
+  if (MODE == 0) step_tail(tail, step_now);
 }
 
 __global__ void sgd_dense_kernel(const DenseParams q, float lr) {
@@ -292,8 +310,8 @@ __global__ void __launch_bounds__(kThreads) sgd_rows_kernel(const RowsParams q, 
   const int64_t n0 = q.tcount[0], total = n0 + q.tcount[1];
   const int64_t wid = (int64_t)blockIdx.x * kWarps + warp, nw = (int64_t)gridDim.x * kWarps;
   for (int64_t e = wid; e < total; e += nw) {
-    const int side = e < n0 ? 0 : 1;
-    const int64_t r = q.list[side][side ? e - n0 : e];
+    const int side = entry_side(e, n0);
+    const int64_t r = entry_row<true>(q, e, n0, side);
     if (q.has_gmf) {
       float* P = q.p_gmf[side] + r * q.f;
       float* G = q.g_gmf[side] + r * q.f;
@@ -317,8 +335,8 @@ __global__ void mark_rows_kernel(const int64_t* __restrict__ user, const int64_t
        b += (int64_t)gridDim.x * blockDim.x) {
     const int64_t u = user[b], it = item[b];
     if (u < 0 || u >= U || it < 0 || it >= I) continue;
-    if (atomicExch(&uflag[u], 1) == 0) ulist[atomicAdd(&tcount[0], 1)] = u;
-    if (atomicExch(&iflag[it], 1) == 0) ilist[atomicAdd(&tcount[1], 1)] = it;
+    claim_row(uflag, ulist, &tcount[0], u);
+    claim_row(iflag, ilist, &tcount[1], it);
   }
 }
 
@@ -343,36 +361,19 @@ __global__ void __launch_bounds__(kThreads) mark_catchup_kernel(const RowsParams
     const int64_t u = user[b], it = item[b];
     if (u < 0 || u >= q.rows[0] || it < 0 || it >= q.rows[1]) continue;   // same rule as mark_rows_kernel
     const int64_t r = side ? it : u;
-    int32_t last = 0;
-    if (lane == 0) {
-      if (atomicExch(&q.flag[side][r], 1) == 0) {
-        (side ? ilist : ulist)[atomicAdd(&tcount[side], 1)] = r;
-        last = q.last[side][r];
-        if (last >= t) last = 0;
-      }
+    // pending_gap's replay-only rule, split around the shuffle: lane 0 clears a current row's `last`.  Called
+    // after the shuffle, the helper changes this kernel's machine code; one such build made the step of batch
+    // 256 6 us slower on a B200 (1000 W limit).
+    int32_t last = 0;   // stays 0 (nothing to replay) in a warp that lost the registration
+    if (lane == 0 && claim_row(q.flag[side], side ? ilist : ulist, &tcount[side], r)) {
+      last = q.last[side][r];
+      if (last >= t) last = 0;
     }
     last = __shfl_sync(0xffffffffu, last, 0);
     if (last <= 0) continue;   // lost the registration, never stepped, or current already
     const int gap = (int)(t - last);
-    __syncwarp();
-    const int n = min(gap, kMaxReplay);
-    for (int j = lane; j < n; j += 32) {
-      const float sj = (float)(last + 1 + j);
-      c1s[j] = bias_c1(q.c, sj);
-      c2s[j] = bias_c2(q.c, sj);
-    }
-    __syncwarp();
-    if (q.has_gmf) {
-      const int64_t o = r * q.f;
-      if (vec) adam_row<4>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, nullptr, q.f, gap, c1s, c2s, 0.f, 0.f, q.c, lane);
-      else adam_row<1>(q.p_gmf[side] + o, q.m_gmf[side] + o, q.v_gmf[side] + o, nullptr, q.f, gap, c1s, c2s, 0.f, 0.f, q.c, lane);
-    }
-    if (q.has_mlp) {
-      const int64_t o = r * q.d;
-      if (vec) adam_row<4>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, nullptr, q.d, gap, c1s, c2s, 0.f, 0.f, q.c, lane);
-      else adam_row<1>(q.p_mlp[side] + o, q.m_mlp[side] + o, q.v_mlp[side] + o, nullptr, q.d, gap, c1s, c2s, 0.f, 0.f, q.c, lane);
-    }
-    if (lane == 0) q.last[side][r] = (int32_t)t;
+    fill_bias_table(c1s, c2s, last, gap, q.c, lane);
+    update_row<false>(q, side, r, gap, vec, c1s, c2s, t, 0.f, 0.f, lane);
   }
 }
 
@@ -384,7 +385,7 @@ __global__ void mark_side_kernel(const int64_t* __restrict__ rows, int64_t n, in
        b += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = rows[b];
     if (r < 0 || r >= limit) continue;
-    if (atomicExch(&flag[r], 1) == 0) list[atomicAdd(count, 1)] = r;
+    claim_row(flag, list, count, r);
   }
 }
 
@@ -421,7 +422,8 @@ __global__ void __launch_bounds__(256) adam_flat_kernel(const FlatParams q) {
     float4 p4 = P[i], m4 = M[i], v4 = V[i];
     const float4 g4 = G[i];
     const int32_t last = __ldg(&T.last[i / T.q4]);
-    const int gap = (last > 0) ? (int)(t - 1 - last) : 0;
+    int gap;
+    pending_gap<true>(last, t - 1, gap);
     float* pp = &p4.x; float* mp = &m4.x; float* vp = &v4.x;
     const float* gp = &g4.x;
 #pragma unroll
@@ -504,8 +506,7 @@ __global__ void __launch_bounds__(256) adam_p2p_kernel(const __grid_constant__ P
   }
 }
 
-__global__ void finalize_step_kernel(int64_t* step, int32_t* tcount) {
-  if (step) *step += 1;
+__global__ void finalize_step_kernel(int32_t* tcount) {
   tcount[0] = 0;
   tcount[1] = 0;
 }
@@ -524,19 +525,61 @@ int rows_grid(int64_t rows) {
   return (int)(blocks < 1 ? 1 : blocks);
 }
 
+// one grid-stride thread per registration (mark kernels)
+int mark_grid(int64_t n) {
+  const int64_t blocks = (n + 255) / 256;
+  return (int)(blocks > 4 * ncf::num_sms() ? 4 * ncf::num_sms() : blocks);
+}
+
 AdamConst make_const(NcfAdamHyper h) { return make_adam_const(h.lr, h.beta1, h.beta2, h.eps); }
 
-void fill_rows(RowsParams& q, const NcfModel* m, const NcfGrads* g, const NcfAdamState* s) {
+int check_hyper(NcfAdamHyper h) {
+  NCF_REQUIRE(h.beta1 > 0.f && h.beta1 < 1.f && h.beta2 > 0.f && h.beta2 < 1.f && h.eps > 0.f,
+              "bad Adam hyper-parameters: need 0 < beta1 < 1, 0 < beta2 < 1 and eps > 0");
+  return NCF_OK;
+}
+
+// Validates an optimiser call: the model and, as `needs` says, the grads, the Adam state, the hyper-parameters.
+enum : int { kGrads = 1, kState = 2, kHyper = 4 };
+int check_call(int needs, const NcfModel* m, const NcfGrads* g, const NcfAdamState* s, NcfAdamHyper h = {}) {
+  int rc = ncf::validate_model(m);
+  if (rc != NCF_OK) return rc;
+  if (needs & kGrads) {
+    NCF_REQUIRE(g && g->g_tower && g->user_flag && g->item_flag && g->user_list && g->item_list &&
+                    g->touched_count,
+                "incomplete NcfGrads");
+    if (m->model_type != NCF_MLP) NCF_REQUIRE(g->g_user_gmf && g->g_item_gmf, "GMF grads are NULL");
+    if (m->model_type != NCF_GMF) NCF_REQUIRE(g->g_user_mlp && g->g_item_mlp, "MLP grads are NULL");
+  }
+  if (needs & kState) {
+    NCF_REQUIRE(s && s->step && s->user_last_step && s->item_last_step && s->m_tower && s->v_tower,
+                "incomplete NcfAdamState");
+    if (m->model_type != NCF_MLP)
+      NCF_REQUIRE(s->m_user_gmf && s->v_user_gmf && s->m_item_gmf && s->v_item_gmf,
+                  "NcfAdamState: GMF moments are NULL");
+    if (m->model_type != NCF_GMF)
+      NCF_REQUIRE(s->m_user_mlp && s->v_user_mlp && s->m_item_mlp && s->v_item_mlp,
+                  "NcfAdamState: MLP moments are NULL");
+  }
+  return (needs & kHyper) ? check_hyper(h) : NCF_OK;
+}
+
+// The preamble of every touched-row entry: check_call, then q filled from what the call takes.
+int rows_call(RowsParams& q, int needs, const NcfModel* m, const NcfGrads* g, const NcfAdamState* s,
+              NcfAdamHyper h = {}) {
+  const int rc = check_call(needs, m, g, s, h);
+  if (rc != NCF_OK) return rc;
+  q = RowsParams{};
   q.p_gmf[0] = m->embed_user_gmf; q.p_gmf[1] = m->embed_item_gmf;
   q.p_mlp[0] = m->embed_user_mlp; q.p_mlp[1] = m->embed_item_mlp;
-  if (g) {
+  if (needs & kGrads) {
     q.g_gmf[0] = g->g_user_gmf; q.g_gmf[1] = g->g_item_gmf;
     q.g_mlp[0] = g->g_user_mlp; q.g_mlp[1] = g->g_item_mlp;
     q.flag[0] = g->user_flag; q.flag[1] = g->item_flag;
     q.list[0] = g->user_list; q.list[1] = g->item_list;
     q.tcount = g->touched_count;
   }
-  if (s) {
+  if (needs & kState) {
     q.m_gmf[0] = s->m_user_gmf; q.m_gmf[1] = s->m_item_gmf;
     q.v_gmf[0] = s->v_user_gmf; q.v_gmf[1] = s->v_item_gmf;
     q.m_mlp[0] = s->m_user_mlp; q.m_mlp[1] = s->m_item_mlp;
@@ -548,6 +591,8 @@ void fill_rows(RowsParams& q, const NcfModel* m, const NcfGrads* g, const NcfAda
   q.f = m->factor_num; q.d = m->mlp_dim;
   q.has_gmf = m->model_type != NCF_MLP;
   q.has_mlp = m->model_type != NCF_GMF;
+  if (needs & kHyper) q.c = make_const(h);
+  return NCF_OK;
 }
 
 void fill_dense(DenseParams& q, const NcfModel* m) {
@@ -562,27 +607,6 @@ void fill_dense(DenseParams& q, const NcfModel* m) {
   q.seg[n++] = {m->predict_w, ts.pw_off, (int64_t)ts.predict_size};
   q.seg[n++] = {m->predict_b, ts.pb_off, 1};
   q.nseg = n;
-}
-
-int check_state(const NcfModel* m, const NcfAdamState* s) {
-  NCF_REQUIRE(s && s->step && s->user_last_step && s->item_last_step && s->m_tower && s->v_tower,
-              "incomplete NcfAdamState");
-  if (m->model_type != NCF_MLP)
-    NCF_REQUIRE(s->m_user_gmf && s->v_user_gmf && s->m_item_gmf && s->v_item_gmf,
-                "NcfAdamState: GMF moments are NULL");
-  if (m->model_type != NCF_GMF)
-    NCF_REQUIRE(s->m_user_mlp && s->v_user_mlp && s->m_item_mlp && s->v_item_mlp,
-                "NcfAdamState: MLP moments are NULL");
-  return NCF_OK;
-}
-
-int check_grads(const NcfModel* m, const NcfGrads* g) {
-  NCF_REQUIRE(g && g->g_tower && g->user_flag && g->item_flag && g->user_list && g->item_list &&
-                  g->touched_count,
-              "incomplete NcfGrads");
-  if (m->model_type != NCF_MLP) NCF_REQUIRE(g->g_user_gmf && g->g_item_gmf, "GMF grads are NULL");
-  if (m->model_type != NCF_GMF) NCF_REQUIRE(g->g_user_mlp && g->g_item_mlp, "MLP grads are NULL");
-  return NCF_OK;
 }
 
 }  // namespace
@@ -612,16 +636,10 @@ extern "C" int ncf_adam_step_dense_range(const NcfModel* m, const NcfGrads* g, c
 
 static int adam_step_impl(const NcfModel* m, const NcfGrads* g, const NcfAdamState* s, NcfAdamHyper h,
                           void* stream, bool all_rows, int64_t user_lo, int64_t user_hi, int parts) {
-  int rc = ncf::validate_model(m);
+  RowsParams q;
+  const int rc = rows_call(q, kGrads | kState | kHyper, m, g, s, h);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
-  if ((rc = check_state(m, s)) != NCF_OK) return rc;
-  NCF_REQUIRE(h.beta1 > 0.f && h.beta1 < 1.f && h.beta2 > 0.f && h.beta2 < 1.f && h.eps > 0.f,
-              "ncf_adam_step: bad hyper-parameters");
   cudaStream_t st = (cudaStream_t)stream;
-  RowsParams q{};
-  fill_rows(q, m, g, s);
-  q.c = make_const(h);
   const bool vec = ((q.f & 3) == 0) && ((q.d & 3) == 0);
   if (all_rows) {  // users [user_lo, user_hi) (data-parallel ranks own a range of the user rows), every item
     q.row0[0] = user_lo;
@@ -671,11 +689,9 @@ static int adam_step_impl(const NcfModel* m, const NcfGrads* g, const NcfAdamSta
 
 static int launch_mark(const NcfModel* m, const NcfGrads* g, const int64_t* user,
                        const int64_t* item, int64_t B, cudaStream_t st) {
-  int64_t blocks = (B + 255) / 256;
-  if (blocks > 4 * ncf::num_sms()) blocks = 4 * ncf::num_sms();
-  mark_rows_kernel<<<(int)blocks, 256, 0, st>>>(user, item, B, m->user_num, m->item_num,
-                                               g->user_flag, g->item_flag, g->user_list,
-                                               g->item_list, g->touched_count);
+  mark_rows_kernel<<<mark_grid(B), 256, 0, st>>>(user, item, B, m->user_num, m->item_num,
+                                                g->user_flag, g->item_flag, g->user_list,
+                                                g->item_list, g->touched_count);
   NCF_LAUNCH_CHECK("mark_rows_kernel");
   g_rows_hint += 2 * B;
   return NCF_OK;
@@ -683,25 +699,21 @@ static int launch_mark(const NcfModel* m, const NcfGrads* g, const int64_t* user
 
 extern "C" int ncf_mark_rows(const NcfModel* m, const NcfGrads* g, const int64_t* user,
                              const int64_t* item, int64_t B, void* stream) {
-  int rc = ncf::validate_model(m);
+  const int rc = check_call(kGrads, m, g, nullptr);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
   NCF_REQUIRE(B > 0 && user && item, "ncf_mark_rows: empty batch or null pointer");
   return launch_mark(m, g, user, item, B, (cudaStream_t)stream);
 }
 
 extern "C" int ncf_mark_rows_side(const NcfModel* m, const NcfGrads* g, const int64_t* rows, int64_t n,
                                   int32_t side, void* stream) {
-  int rc = ncf::validate_model(m);
+  const int rc = check_call(kGrads, m, g, nullptr);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
   NCF_REQUIRE(side == 0 || side == 1, "ncf_mark_rows_side: side must be 0 (users) or 1 (items)");
   NCF_REQUIRE(n >= 0, "ncf_mark_rows_side: negative n");
   if (n == 0) return NCF_OK;
   NCF_REQUIRE(rows != nullptr, "ncf_mark_rows_side: rows is NULL");
-  int64_t blocks = (n + 255) / 256;
-  if (blocks > 4 * ncf::num_sms()) blocks = 4 * ncf::num_sms();
-  mark_side_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+  mark_side_kernel<<<mark_grid(n), 256, 0, (cudaStream_t)stream>>>(
       rows, n, side ? m->item_num : m->user_num, side ? g->item_flag : g->user_flag,
       side ? g->item_list : g->user_list, g->touched_count + side);
   NCF_LAUNCH_CHECK("mark_side_kernel");
@@ -711,13 +723,9 @@ extern "C" int ncf_mark_rows_side(const NcfModel* m, const NcfGrads* g, const in
 
 extern "C" int ncf_adam_catchup(const NcfModel* m, const NcfGrads* g, const NcfAdamState* s,
                                 NcfAdamHyper h, void* stream) {
-  int rc = ncf::validate_model(m);
+  RowsParams q;
+  const int rc = rows_call(q, kGrads | kState | kHyper, m, g, s, h);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
-  if ((rc = check_state(m, s)) != NCF_OK) return rc;
-  RowsParams q{};
-  fill_rows(q, m, g, s);
-  q.c = make_const(h);
   adam_rows_kernel<2><<<rows_grid(g_rows_hint), kThreads, 0, (cudaStream_t)stream>>>(q, StepTail{});
   NCF_LAUNCH_CHECK("adam_rows_kernel<catchup>");
   return NCF_OK;
@@ -726,22 +734,16 @@ extern "C" int ncf_adam_catchup(const NcfModel* m, const NcfGrads* g, const NcfA
 extern "C" int ncf_adam_prepare(const NcfModel* m, const NcfGrads* g, const NcfAdamState* s,
                                 NcfAdamHyper h, const int64_t* user, const int64_t* item, int64_t B,
                                 void* stream) {
-  int rc = ncf::validate_model(m);
+  RowsParams q;
+  int rc = rows_call(q, kGrads | kState | kHyper, m, g, s, h);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
-  if ((rc = check_state(m, s)) != NCF_OK) return rc;
   NCF_REQUIRE(B > 0 && user && item, "ncf_adam_prepare: empty batch or null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  RowsParams q{};
-  fill_rows(q, m, g, s);
-  q.c = make_const(h);
   if (B > 4096) {
     // large batches: a thread per sample registers (one warp per sample-side would serialise 2B dependent
     // chains on a few thousand resident warps), then a warp per DISTINCT row replays
     if ((rc = launch_mark(m, g, user, item, B, st)) != NCF_OK) return rc;
-    adam_rows_kernel<2><<<rows_grid(g_rows_hint), kThreads, 0, st>>>(q, StepTail{});
-    NCF_LAUNCH_CHECK("adam_rows_kernel<catchup>");
-    return NCF_OK;
+    return ncf_adam_catchup(m, g, s, h, stream);
   }
   mark_catchup_kernel<<<rows_grid(2 * B), kThreads, 0, st>>>(q, user, item, B, g->user_list, g->item_list,
                                                              g->touched_count);
@@ -752,24 +754,19 @@ extern "C" int ncf_adam_prepare(const NcfModel* m, const NcfGrads* g, const NcfA
 
 extern "C" int ncf_adam_flush(const NcfModel* m, const NcfAdamState* s, NcfAdamHyper h,
                               void* stream) {
-  int rc = ncf::validate_model(m);
+  RowsParams q;
+  const int rc = rows_call(q, kState | kHyper, m, nullptr, s, h);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_state(m, s)) != NCF_OK) return rc;
-  RowsParams q{};
-  fill_rows(q, m, nullptr, s);
-  q.c = make_const(h);
   adam_rows_kernel<1><<<ncf::num_sms() * 8, kThreads, 0, (cudaStream_t)stream>>>(q, StepTail{});
   NCF_LAUNCH_CHECK("adam_rows_kernel<flush>");
   return NCF_OK;
 }
 
 extern "C" int ncf_sgd_step(const NcfModel* m, const NcfGrads* g, float lr, void* stream) {
-  int rc = ncf::validate_model(m);
+  RowsParams q;
+  const int rc = rows_call(q, kGrads, m, g, nullptr);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  RowsParams q{};
-  fill_rows(q, m, g, nullptr);
   sgd_rows_kernel<<<rows_grid(g_rows_hint), kThreads, 0, st>>>(q, lr);
   g_rows_hint = 0;
   NCF_LAUNCH_CHECK("sgd_rows_kernel");
@@ -778,7 +775,7 @@ extern "C" int ncf_sgd_step(const NcfModel* m, const NcfGrads* g, float lr, void
   dq.g = g->g_tower;
   sgd_dense_kernel<<<dim3(32, dq.nseg), 256, 0, st>>>(dq, lr);
   NCF_LAUNCH_CHECK("sgd_dense_kernel");
-  finalize_step_kernel<<<1, 1, 0, st>>>(nullptr, g->touched_count);
+  finalize_step_kernel<<<1, 1, 0, st>>>(g->touched_count);
   NCF_LAUNCH_CHECK("finalize_step_kernel");
   return NCF_OK;
 }
@@ -790,8 +787,8 @@ extern "C" int ncf_adam_range(float* p, float* m, float* v, float* g, int64_t n,
   NCF_REQUIRE(n >= 0 && (n & 3) == 0, "ncf_adam_range: n must be a multiple of 4");
   NCF_REQUIRE((((uintptr_t)p | (uintptr_t)m | (uintptr_t)v | (uintptr_t)g) & 15) == 0,
               "ncf_adam_range: pointers must be 16-byte aligned");
-  NCF_REQUIRE(h.beta1 > 0.f && h.beta1 < 1.f && h.beta2 > 0.f && h.beta2 < 1.f && h.eps > 0.f,
-              "ncf_adam_range: bad hyper-parameters");
+  const int rc = check_hyper(h);
+  if (rc != NCF_OK) return rc;
   if (n == 0) return NCF_OK;
   adam_range_kernel<<<ncf::num_sms() * 8, 256, 0, (cudaStream_t)stream>>>(
       reinterpret_cast<float4*>(p), reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v),
@@ -807,8 +804,8 @@ extern "C" int ncf_adam_p2p(const void* const* grad_bufs, void* const* param_buf
   NCF_REQUIRE(world >= 1 && world <= 8 && rank >= 0 && rank < world, "ncf_adam_p2p: world must be 1..8 (one node)");
   NCF_REQUIRE(lo >= 0 && n >= 0 && (lo & 3) == 0 && (n & 3) == 0, "ncf_adam_p2p: lo and n must be multiples of 4");
   NCF_REQUIRE((((uintptr_t)m | (uintptr_t)v) & 15) == 0, "ncf_adam_p2p: pointers must be 16-byte aligned");
-  NCF_REQUIRE(h.beta1 > 0.f && h.beta1 < 1.f && h.beta2 > 0.f && h.beta2 < 1.f && h.eps > 0.f,
-              "ncf_adam_p2p: bad hyper-parameters");
+  const int rc = check_hyper(h);
+  if (rc != NCF_OK) return rc;
   PeerBufs b{};
   for (int r = 0; r < world; ++r) {
     NCF_REQUIRE(grad_bufs[r] && param_bufs[r], "ncf_adam_p2p: null peer buffer");
@@ -826,10 +823,8 @@ extern "C" int ncf_adam_p2p(const void* const* grad_bufs, void* const* param_buf
 }
 
 extern "C" int ncf_adam_finish_dense(const NcfModel* m, const NcfGrads* g, const NcfAdamState* s, void* stream) {
-  int rc = ncf::validate_model(m);
+  const int rc = check_call(kGrads | kState, m, g, s);
   if (rc != NCF_OK) return rc;
-  if ((rc = check_grads(m, g)) != NCF_OK) return rc;
-  if ((rc = check_state(m, s)) != NCF_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   StepTail tail{};
   tail.step = s->step;

@@ -222,7 +222,7 @@ __global__ void shard_mark_requests_kernel(const int64_t* __restrict__ inbox, co
     if (j >= cnt[r]) continue;
     const int64_t row = inbox[e] >> 32;
     if (row < 0 || row >= limit) continue;
-    if (atomicExch(&flag[row], 1) == 0) list[atomicAdd(count, 1)] = row;
+    claim_row(flag, list, count, row);
   }
 }
 

@@ -16,16 +16,12 @@ import pytest
 import torch
 
 from oracle import ncf_numpy as onp
-from tests.util import assert_close
+from tests.util import HYPER, REPLAY, adam_ref, assert_adam, assert_close, lazy_ref
 
 gpu = pytest.mark.gpu
 
 ERR_ARG = -1
-LR, B1, B2, EPS = 1e-3, 0.9, 0.999, 1e-8
-# the optimiser kernels receive fp32 hyper-parameters; the float64 references use exactly those values
-HYPER = tuple(float(np.float32(x)) for x in (LR, B1, B2, EPS))
 STEPS = [0, 1, 4, 999]   # step counters before the call; at 999 an off-by-one bias correction moves p by ~3e-4
-REPLAY = 160             # exact zero-gradient steps replayed per row (adam_math.cuh kMaxReplay, DESIGN §3.2)
 
 
 def _dev():
@@ -60,34 +56,6 @@ def _ptrs(addresses):
 
 
 # ---- float64 references ----------------------------------------------------------------------------------------
-def adam_ref(p, m, v, g, t, hyper=HYPER):
-    """torch.optim.Adam, one step at step index t (1-based), in float64 (adam_math.cuh)."""
-    lr, b1, b2, eps = hyper
-    p, m, v, g = (np.asarray(x, np.float64) for x in (p, m, v, g))
-    m = m + (1 - b1) * (g - m)
-    v = b2 * v + (1 - b2) * g * g
-    p = p - lr / (1 - b1 ** t) * m / (np.sqrt(v) / np.sqrt(1 - b2 ** t) + eps)
-    return p, m, v
-
-
-def lazy_ref(p, m, v, g, last, t, hyper=HYPER):
-    """The all-rows step t of a row last stepped at `last` (0 = never, treated as current): replay the
-    min(gap, 160) zero-gradient steps last+1 .. exactly, decay m and v by beta^gap in closed form, then take
-    the real step t (DESIGN §3.2).  p, m, v, g: [rows, dim]; last: [rows].  Returns (p, m, v, gap)."""
-    lr, b1, b2, eps = hyper
-    p, m, v = (np.asarray(x, np.float64).copy() for x in (p, m, v))
-    last = np.asarray(last, np.int64)[:, None]
-    gap = np.where(last > 0, t - 1 - last, 0)
-    n = np.minimum(gap, REPLAY)
-    for j in range(1, int(n.max(initial=0)) + 1):
-        s = last + j
-        term = lr / (1 - b1 ** s) * (m * b1 ** j) / (np.sqrt(v) * np.sqrt(b2) ** j / np.sqrt(1 - b2 ** s) + eps)
-        p -= np.where(j <= n, term, 0.0)
-    m, v = m * b1 ** gap, v * b2 ** gap
-    p, m, v = adam_ref(p, m, v, g, t, hyper)
-    return p, m, v, np.broadcast_to(gap, p.shape)
-
-
 def bucket_ref(item, world):
     """(owner, local index) of every sample: owner item % world, local item // world; a negative item goes
     to owner 0 with local index -1."""
@@ -114,33 +82,20 @@ def sum_bound(k, abs_sum):
     return k * 2.0 ** -24 * abs_sum
 
 
-def assert_adam(p, p_ref, p_before, m, m_ref, v, v_ref, what, chained=None):
-    """p within one final rounding plus 1e-5 of the step; m / v within 1e-6 of each tensor's largest
-    element.  `chained` (optional, per element): zero-gradient steps the kernel replayed before the real one.
-    Each of them rounds p once more in fp32, so such elements get chained * 2^-24 * |p| on top."""
-    p, p_ref, p_before = (np.asarray(x, np.float64) for x in (p, p_ref, p_before))
-    bar = 2.0 ** -23 * np.abs(p_ref) + 1e-5 * np.abs(p_ref - p_before)
-    if chained is not None:
-        bar = bar + np.minimum(chained, REPLAY) * 2.0 ** -24 * np.maximum(np.abs(p_ref), np.abs(p_before))
-    err = np.abs(p - p_ref)
-    bad = err > bar
-    assert not bad.any(), (f"{what}: p off at {int(bad.sum())}/{bad.size} elements, worst err/bar "
-                           f"{float((err / np.maximum(bar, 1e-300)).max()):.3g}")
-    for name, a, r in (("m", m, m_ref), ("v", v, v_ref)):
-        a, r = np.asarray(a, np.float64), np.asarray(r, np.float64)
-        scale = max(float(np.abs(r).max(initial=0.0)), 1e-30)
-        e = float(np.abs(a - r).max(initial=0.0)) / scale
-        assert e <= 1e-6, f"{what}: {name} relative error {e:.3e} > 1e-6"
-
-
 # ---- CPU: the references against literal loops -----------------------------------------------------------------
-@pytest.mark.parametrize("last,t", [(5, 100), (37, 198), (1, 162), (3, 400), (12, 700), (250, 500), (0, 50), (99, 100)])
-def test_lazy_reference_matches_dense_adam_step_by_step(monkeypatch, last, t):
+_LAZY_STEP = [(5, 100), (37, 198), (1, 162), (3, 400), (12, 700), (250, 500), (0, 50), (99, 100)]
+_LAZY_REPLAY = _LAZY_STEP + [(100, 100), (120, 100)]
+
+
+@pytest.mark.parametrize("last,t,step", [(a, b, True) for a, b in _LAZY_STEP] + [(a, b, False) for a, b in _LAZY_REPLAY],
+                         ids=[f"{a}-{b}" for a, b in _LAZY_STEP] + [f"{a}-{b}-replay" for a, b in _LAZY_REPLAY])
+def test_lazy_reference_matches_dense_adam_step_by_step(monkeypatch, last, t, step):
     """lazy_ref == oracle DenseAdam run step by step with zero gradients from step last+1 to t-1, then with
-    the real gradient at step t.  DenseAdam is run in float64 (its fp32 casts patched out) so that only the
-    truncation of the replay remains: DESIGN §3.2 bounds the terms dropped beyond 160 steps, all together, by
-    1.4e-6 of the first replayed term (the largest ratio, 1.39e-6, is at last = 12; the bias corrections make
-    early rows decay slower than (b1/sqrt(b2))^j)."""
+    the real gradient at step t.  Replay only (step=False, catch-up and flush): zero gradients from step last+1
+    to t and no real step, nothing at all for last = 0 or last >= t.  DenseAdam is run in float64 (its fp32
+    casts patched out) so that only the truncation of the replay remains: DESIGN §3.2 bounds the terms dropped
+    beyond 160 steps, all together, by 1.4e-6 of the first replayed term (the largest ratio, 1.39e-6, is at
+    last = 12; the bias corrections make early rows decay slower than (b1/sqrt(b2))^j)."""
     monkeypatch.setattr(onp, "F32", np.float64)
     rng = np.random.default_rng(last * 1000 + t)
     p0 = rng.standard_normal((4, 6)) * 0.1
@@ -151,16 +106,19 @@ def test_lazy_reference_matches_dense_adam_step_by_step(monkeypatch, last, t):
     lr, b1, b2, eps = HYPER
     opt = onp.DenseAdam(lr, b1, b2, eps)
     params = {"w": p0.copy()}
+    replay = last > 0 and (step or last < t)
     # last = 0 (never stepped) counts as current: the real step is step t
     opt.state["w"] = {"t": last if last > 0 else t - 1, "m": m0.copy(), "v": v0.copy()}
-    if last > 0:
-        for _ in range(last + 1, t):
+    if replay:
+        for _ in range(last + 1, t if step else t + 1):
             opt.step(params, {"w": np.zeros_like(p0)})
-    opt.step(params, {"w": g})
-    p, m, v, gap = lazy_ref(p0, m0, v0, g, np.full(4, last), t)
-    assert int(gap.max()) == (t - 1 - last if last > 0 else 0)
+    if step:
+        opt.step(params, {"w": g})
+    p, m, v, gap = lazy_ref(p0, m0, v0, g if step else None, np.full(4, last), t, step=step)
+    want_gap = (t - 1 - last if step else t - last) if replay else 0
+    assert int(gap.max()) == int(gap.min()) == want_gap
     first = lr / (1 - b1 ** (last + 1)) * np.abs(m0) * b1 / (np.sqrt(v0 * b2) / np.sqrt(1 - b2 ** (last + 1)) + eps)
-    tail = 1.4e-6 * first if last > 0 and t - 1 - last > REPLAY else 0.0
+    tail = 1.4e-6 * first if want_gap > REPLAY else 0.0
     assert np.all(np.abs(p - params["w"]) <= tail + 1e-12 * np.abs(p0) + 1e-15)
     assert np.allclose(m, opt.state["w"]["m"], rtol=1e-12, atol=0)
     assert np.allclose(v, opt.state["w"]["v"], rtol=1e-12, atol=0)
